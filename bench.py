@@ -20,6 +20,10 @@ are real MYULA warm-up iterations (Guassian.m:78-91) and are not timed.
   --impl reference : the CPU restatement of the reference (oracle/, numpy +
           scipy.fft on all host cores + the plain-C TV prox) timed on REAL
           iterations at --size: one chain, K steps after W warm-up steps.
+  --dump-outputs DIR : after the timed steps, writes what the device-timed main
+          loop returned (its trajectories and a seeded sample of every chain's
+          last sample) as DIR/<name>.npy in float64, so that two builds can be
+          compared output for output on identical inputs.
 
 At N = 1 the line also carries (extra keys) the other BASELINE.json configs:
 configs[0] the full run_Gaussian_demo.m run on cameraman 256^2, configs[1]
@@ -46,6 +50,11 @@ CHAMBOLLE_K = 25                 # run_Gaussian_demo.m:188
 EVMAX = 0.993                    # evMax of A'A at (w1,w2)=(1,1): what the reference's power iteration returns
 UNIT = "chain-steps/s"
 METRIC = "MYULA chain-iterations/sec"
+# --dump-outputs: trajectories of the timed main loop besides thetas / sigmas / chambolle_iters, and how many values of
+# the chains' last samples are kept (all chains of the rank and the pixel indices together: 32 MiB in float64)
+DUMP_TRACES = ("psi0", "psi1", "grad_theta", "grad_psi0", "grad_psi1", "grad_sigma", "logPiTraceX", "gXTrace")
+DUMP_LAST_SAMPLE_VALUES = 1 << 22
+DUMP_SEED = 0
 
 
 def alg_bytes_per_chain_step(npix, k=CHAMBOLLE_K):
@@ -62,6 +71,19 @@ def synthetic_truth(n):
     cm = np.load(golden("cman_u8.npy")).astype(np.float64)
     reps = (n + 255) // 256
     return np.tile(cm, (reps, reps))[:n, :n].copy()
+
+
+def last_sample_pixels(npix, nch, seed=DUMP_SEED):
+    """Sorted pixel indices (column-major, as the device holds an image) at which --dump-outputs keeps every chain's
+    last sample: a fixed, seeded choice that depends on the image size and the number of chains only."""
+    per = max(1, min(npix, DUMP_LAST_SAMPLE_VALUES // (nch + 1)))        # nch rows of values + the index row
+    return np.sort(np.random.default_rng(seed).choice(npix, per, replace=False))
+
+
+def write_dump(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def gaussian_op(n, sigma, sigma_min, sigma_max, evMax, samples, warmup):
@@ -338,6 +360,9 @@ def run_ours(args, rank, world, local_rank):
     th = np.zeros(K + 1); tr.thetas = th.ctypes.data_as(c_double_p)
     s2 = np.zeros(K + 1); tr.sigmas = s2.ctypes.data_as(c_double_p)
     ck = np.zeros(K + 1, dtype=np.int32); tr.chambolle_iters = ck.ctypes.data_as(C.POINTER(C.c_int32))
+    dump = {f: np.zeros(K + 1) for f in DUMP_TRACES} if args.dump_outputs else {}
+    for f, b in dump.items():                                 # copied back after the clock stops
+        setattr(tr, f, b.ctypes.data_as(c_double_p))
     barrier()
     clocks = ClockSampler(local_rank) if rank == 0 else None
     rc = lib.sbd_sapg_run_dev(eng._h, y_dev.data_ptr(), None, C.byref(prm), C.byref(tr))
@@ -347,6 +372,24 @@ def run_ours(args, rank, world, local_rank):
     clk = clocks.stop() if clocks else None
     t_main = max_over_ranks(tr.seconds_main)
     launches = int(tr.launches_main)
+    if args.dump_outputs:
+        # The timed run leaves the chains' last samples on the device.  The same run (same inputs, seed and summation
+        # order, so bit-identical) is repeated untimed with their copy-out switched on, and must reproduce the timed
+        # trajectories.
+        xl = torch.empty(nch * npix, dtype=torch.float64).pin_memory()
+        tr_x = sbd_traces()
+        th_x = np.zeros(K + 1); tr_x.thetas = th_x.ctypes.data_as(c_double_p)
+        s2_x = np.zeros(K + 1); tr_x.sigmas = s2_x.ctypes.data_as(c_double_p)
+        tr_x.X_last = C.cast(xl.data_ptr(), c_double_p)
+        rc = lib.sbd_sapg_run_dev(eng._h, y_dev.data_ptr(), None, C.byref(prm), C.byref(tr_x))
+        if rc != 0:
+            raise RuntimeError(lib.sbd_last_error(eng._h).decode())
+        if not (np.array_equal(th_x, th) and np.array_equal(s2_x, s2)):
+            raise RuntimeError("--dump-outputs: the repeated main loop did not reproduce the timed one")
+        idx = last_sample_pixels(npix, nch)
+        dump.update(thetas=th, sigmas=s2, chambolle_iters=ck, X_last_sample_index=idx,
+                    X_last_sample=xl.numpy().reshape(nch, npix)[:, idx])
+        del xl
     # per-phase CUDA-event times come from a second, short run with the phase timers on: profiling serialises the
     # two streams of an iteration (prox next to analysis + gradient), so it is kept out of the headline number
     KP = min(K, 4)
@@ -444,6 +487,8 @@ def run_ours(args, rank, world, local_rank):
         line["cpu_baseline"] = {"value": rate, "unit": UNIT, "cores": workers, "kind": "port",
                                 "s_per_iteration": [round(float(p), 3) for p in per],
                                 "sample": cpu_sample_text(n, cs, cw, workers)}
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, dump)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -607,7 +652,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[0]/[1]/[2]/[4] extra keys")
     ap.add_argument("--cman-samples", type=int, default=20000)
     ap.add_argument("--cman-warmup", type=int, default=15000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed main loop's trajectories and a seeded sample of its chains' last samples "
+                         "as DIR/<name>.npy (float64; the sample and its indices take 32 MiB at most)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

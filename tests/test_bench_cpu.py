@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -49,3 +51,22 @@ def test_chain_split_is_strong_scaling():
     assert bench.chains_for(a, 4) == (8, 32) and bench.scaling_kind(a) == "weak"
     assert bench.alg_bytes_per_chain_step(4096 * 4096) == 1144 * 4096 * 4096
     assert bench.chamb_plan_n4(25) == 4 and bench.chamb_plan_n4(20) == 4
+
+
+def test_dump_sample_is_fixed_and_bounded():
+    """--dump-outputs keeps the chains' last samples at seeded pixels: the same for every run, within 32 MiB (float64)
+    with the index row, and every pixel when the image is small."""
+    sys.path.insert(0, ROOT)
+    import bench
+    for npix, nch in ((4096 * 4096, 64), (4096 * 4096, 1), (2048 * 2048, 8)):
+        idx = bench.last_sample_pixels(npix, nch)
+        assert np.array_equal(idx, bench.last_sample_pixels(npix, nch))
+        assert idx[0] >= 0 and idx[-1] < npix and np.all(np.diff(idx) > 0)
+        assert (nch + 1) * idx.size * 8 <= 32 << 20
+    assert np.array_equal(bench.last_sample_pixels(256 * 256, 8), np.arange(256 * 256))
+
+
+def test_dump_outputs_is_for_the_gpu_arm():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", "x"],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr
