@@ -40,7 +40,7 @@ extern "C" {
 #define SBD_E_NODEVICE   -3   /* no usable GPU                                        */
 #define SBD_E_NOMEM      -4   /* device allocation failed                             */
 #define SBD_E_COMM       -5   /* NCCL error / communicator not initialised            */
-#define SBD_E_UNSUPPORTED -6  /* e.g. FFT operators on a non power-of-two size         */
+#define SBD_E_UNSUPPORTED -6  /* e.g. FFT operators on a side with a prime factor > 7  */
 
 /* PSF families.  psi = (w1,w2) | (alpha,beta) | (b,-) */
 #define SBD_GAUSSIAN 0        /* utils/Gaussian_psf.m:2-19   */
@@ -62,8 +62,10 @@ typedef struct sbd_ctx sbd_ctx;
 
 /* ------------------------------------------------------------------------
  * Context.  rows x cols is the image size (MATLAB size(x)); the FFT-based
- * operators need both to be powers of two in [16, 4096]; the TV entry points
- * (tvnorm, diffh/diffv, tvprox) accept any size >= 2.  `max_batch` is the
+ * operators take every size whose sides lie in [max(psf_size, 2), 4096] and
+ * have no prime factor above 7 (other sizes: SBD_E_UNSUPPORTED, naming the
+ * side and its factor); the TV entry points (tvnorm, diffh/diffv, tvprox)
+ * accept any size >= 2.  `max_batch` is the
  * largest number of images / Markov chains a single call will carry.
  * ---------------------------------------------------------------------- */
 int sbd_create(sbd_ctx** out, int rows, int cols, int psf_size, int model,

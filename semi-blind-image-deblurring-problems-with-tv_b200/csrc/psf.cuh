@@ -92,7 +92,7 @@ __global__ void k_psf_colcoef(int t, int nx, int nk, const double* __restrict__ 
     const double* h = taps + (size_t)m * t * t + (size_t)j * t;
     double re = 0.0, im = 0.0;
     for (int i = 0; i < t; ++i) {
-        const double2 w = tw_nx[(int)(((long long)k * i) & (nx - 1))];
+        const double2 w = tw_nx[(int)(((long long)k * i) % nx)];
         re = fma(h[i], w.x, re);
         im = fma(h[i], w.y, im);
     }
@@ -213,7 +213,7 @@ __global__ void k_psf_spectrum(int t, int nx, int ny, int m, const double2* __re
     const double2* a = coef + ((size_t)m * nx + k) * MAXT;
     double sr = 0.0, si = 0.0;
     for (int j = 0; j < t; ++j) {
-        const double2 w = tw_ny[(int)(((long long)q * j) & (ny - 1))];
+        const double2 w = tw_ny[(int)(((long long)q * j) % ny)];
         const double2 p = cmul(a[j], w);
         sr += p.x; si += p.y;
     }

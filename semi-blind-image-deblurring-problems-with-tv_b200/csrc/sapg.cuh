@@ -15,7 +15,9 @@
 namespace sbd {
 
 // X <- | X + gam*(P - X)/lamb - gam*Gf + sqrt(2 gam) Z |   (two elements per thread)
-// grid = (ceil(npix/2/blockDim), n_chains)
+// grid = (ceil(ceil(npix/2)/blockDim), n_chains)
+// An odd npix puts the element pairs of every other chain off the 16-byte grid: scalar accesses there, and the last
+// element of an image (a pair of its own) takes z0 of its pair (oracle/philox.py).
 __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
                            const double* __restrict__ Gf, const double* __restrict__ noise,
                            double* __restrict__ post_mean, const Control* __restrict__ ctl,
@@ -26,6 +28,28 @@ __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
     const int ch = blockIdx.y;
     const size_t off = (size_t)ch * npix + 2 * pair;
     const unsigned int draw = ctl->draw;
+    if (npix & 1) {
+        const bool two = 2 * pair + 1 < npix;
+        double2 z;
+        if (noise) {
+            const double* nz = noise + ((size_t)draw * n_chains + ch) * npix + 2 * pair;
+            z = make_double2(__ldg(nz), two ? __ldg(nz + 1) : 0.0);
+        } else {
+            z = philox_normal2(seed, (uint32_t)(chain_offset + ch), draw, pair);
+        }
+        const int ne = two ? 2 : 1;
+        const bool acc = post_mean && ctl->phase == 1 && ctl->ii > burnIn;
+        for (int e = 0; e < ne; ++e) {
+            const double x = X[off + e], p = __ldg(P + off + e), gf = __ldg(Gf + off + e), ze = e ? z.y : z.x;
+            const double r = fabs(((x + (gam * (p - x)) / lamb) - gam * gf) + sq2gam * ze);
+            X[off + e] = r;
+            if (acc) {
+                const double inv = 1.0 / (double)(ctl->ii - burnIn);
+                post_mean[off + e] += (r - post_mean[off + e]) * inv;
+            }
+        }
+        return;
+    }
     double2 z;
     if (noise) {
         z = __ldg(reinterpret_cast<const double2*>(noise + ((size_t)draw * n_chains + ch) * npix + 2 * pair));
@@ -252,6 +276,14 @@ __global__ void k_add_noise(const double* __restrict__ ax, const double* __restr
                             double* __restrict__ y, size_t npix, uint64_t seed, uint32_t stream) {
     const size_t pair = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (2 * pair >= npix) return;
+    if (npix & 1) {                 // the last element of an odd image takes z0 of its pair
+        const bool two = 2 * pair + 1 < npix;
+        const double2 z = noise ? make_double2(noise[2 * pair], two ? noise[2 * pair + 1] : 0.0)
+                                : philox_normal2(seed, stream, 0u, pair);
+        y[2 * pair] = ax[2 * pair] + sigma * z.x;
+        if (two) y[2 * pair + 1] = ax[2 * pair + 1] + sigma * z.y;
+        return;
+    }
     double2 z;
     if (noise) z = *reinterpret_cast<const double2*>(noise + 2 * pair);
     else z = philox_normal2(seed, stream, 0u, pair);
@@ -263,6 +295,11 @@ __global__ void k_philox_image(double* __restrict__ x, size_t npix, uint64_t see
     const size_t pair = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (2 * pair >= npix) return;
     const double2 z = philox_normal2(seed, stream, 0u, pair);
+    if (npix & 1) {                 // odd image: the last element takes z0 of its pair
+        x[2 * pair] = z.x;
+        if (2 * pair + 1 < npix) x[2 * pair + 1] = z.y;
+        return;
+    }
     *reinterpret_cast<double2*>(x + 2 * pair) = z;
 }
 

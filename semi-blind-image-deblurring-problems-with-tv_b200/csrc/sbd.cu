@@ -11,6 +11,7 @@
 #include "tv_coop.cuh"
 #include "fft.cuh"
 #include "fft2.cuh"
+#include "fft_any.cuh"
 #include "sapg.cuh"
 
 #include <dlfcn.h>
@@ -66,7 +67,10 @@ struct sbd_ctx {
     int t = 7, model = 0;
     double phi = 0.0;
     int max_batch = 1;
-    bool pow2 = false;
+    bool pow2 = false;              // FFT passes of fft.cuh / fft2.cuh
+    bool smooth = false;            // every other size the FFT operators take: fft_any.cuh (fft_plan.h)
+    std::string fft_err;            // why the FFT operators refuse this size ("" when they take it)
+    AnyPlan plan_x = {}, plan_y = {};   // smooth: plans of the rows (length nx) and column (length ny) passes
     size_t npix = 0;
     int sp = 0, nk = 0;             // half-spectrum pitch / number of bins (nx/2+1)
     size_t spec_elems = 0;          // per image, in double2
@@ -176,8 +180,8 @@ void make_twiddles(int n, double2* d, cudaStream_t s) {
         h[m].x = (double)cosl(a);
         h[m].y = (double)sinl(a);
     }
-    if (n >= 4) { h[n / 4] = make_double2(0.0, -1.0); h[n / 2] = make_double2(-1.0, 0.0); h[3 * n / 4] = make_double2(0.0, 1.0); }
-    else if (n == 2) h[1] = make_double2(-1.0, 0.0);
+    if (n % 4 == 0) { h[n / 4] = make_double2(0.0, -1.0); h[n / 2] = make_double2(-1.0, 0.0); h[3 * n / 4] = make_double2(0.0, 1.0); }
+    else if (n % 2 == 0) h[n / 2] = make_double2(-1.0, 0.0);
     SBD_CUDA(cudaMemcpyAsync(d, h.data(), sizeof(double2) * n, cudaMemcpyHostToDevice, s));
     SBD_CUDA(cudaStreamSynchronize(s));
 }
@@ -281,7 +285,7 @@ void ensure_ws(sbd_ctx* c, int batch) {
     const size_t n = (size_t)batch * c->npix;
     c->X = dalloc<double>(n); c->P = dalloc<double>(n); c->Gf = dalloc<double>(n);
     c->px0 = dalloc<double>(n); c->py0 = dalloc<double>(n); c->px1 = dalloc<double>(n); c->py1 = dalloc<double>(n);
-    if (c->pow2) {
+    if (c->pow2 || c->smooth) {
         c->S1 = dalloc<double2>((size_t)batch * c->spec_elems);
         c->S2 = dalloc<double2>((size_t)batch * c->spec_elems);
         if (c->v2) { c->tm_S1 = make_spec_tmap(c, c->S1, batch); c->tm_S2 = make_spec_tmap(c, c->S2, batch); }
@@ -563,7 +567,20 @@ SpecGeom spec_geom(const sbd_ctx* c) {
 
 #define SBD_FFT2_SIZES(X) X(1024) X(2048) X(4096)
 
+// The mixed-radix kernels serve every size with one instantiation, and the dynamic shared-memory limit is a property of
+// the kernel on the device, not of a context: each opts in once to the largest line any size needs (ANY_MAXN double2),
+// so that no context can lower the limit under another one that uses a longer line.
+constexpr size_t ANY_SMEM_OPTIN = (size_t)ANY_MAXN * sizeof(double2);
+
 void rows_fwd(sbd_ctx* c, const double* x, double2* spec, int batch) {
+    if (c->smooth) {
+        const size_t smem = (size_t)c->nx * 16;
+        set_smem(c, k_rows_any_fwd, ANY_SMEM_OPTIN);
+        k_rows_any_fwd<<<dim3((c->ny + 1) / 2, batch), c->plan_x.T, smem, c->stream>>>(x, spec, c->plan_x, c->ny, c->npix,
+                                                                                       c->spec_elems, c->tw_nx);
+        LAUNCH_CHECK(c);
+        return;
+    }
     if (c->v2) {
         const size_t smem2 = (size_t)c->nx * 16;
         dim3 g2(c->ny / 2, batch);
@@ -593,6 +610,14 @@ void rows_fwd(sbd_ctx* c, const double* x, double2* spec, int batch) {
 }
 
 void rows_inv(sbd_ctx* c, const double2* spec, double* out, int batch) {
+    if (c->smooth) {
+        const size_t smem = (size_t)c->nx * 16;
+        set_smem(c, k_rows_any_inv, ANY_SMEM_OPTIN);
+        k_rows_any_inv<<<dim3((c->ny + 1) / 2, batch), c->plan_x.T, smem, c->stream>>>(spec, out, c->plan_x, c->ny, c->npix,
+                                                                                       c->spec_elems, c->tw_nx);
+        LAUNCH_CHECK(c);
+        return;
+    }
     if (c->v2) {
         const size_t smem2 = (size_t)c->nx * 16;
         dim3 g2(c->ny / 2, batch);
@@ -630,6 +655,13 @@ void cols(sbd_ctx* c, const double2* in, double2* out, int batch, int opsel = 0)
     a.nsub = c->colsC / c->colsKC; a.ntiles = c->ntiles; a.opsel = opsel;
     a.opscale = 1.0 / ((double)c->nx * (double)c->ny);
     a.mu = c->salsa_mu;
+    if (c->smooth) {
+        const size_t smem = (size_t)c->ny * 16;
+        set_smem(c, k_cols_any<MODE>, ANY_SMEM_OPTIN);
+        k_cols_any<MODE><<<dim3(batch, c->nk), c->plan_y.T, smem, c->stream>>>(a, c->plan_y);
+        LAUNCH_CHECK(c);
+        return;
+    }
     if (c->v2) {
         const size_t smem2 = (size_t)c->ny * 16;
         dim3 g2(batch, c->nk);
@@ -672,9 +704,8 @@ void psf_from_host(sbd_ctx* c, const double psi[2], int nkc) {
     if (nkc > 0) psf_refresh_coef(c, nkc);
 }
 
-void require_pow2(sbd_ctx* c) {
-    SBD_REQUIRE(c->pow2, SBD_E_UNSUPPORTED,
-                "FFT operators need rows and cols to be powers of two in [16, 4096]");
+void require_fft(sbd_ctx* c) {
+    SBD_REQUIRE(c->pow2 || c->smooth, SBD_E_UNSUPPORTED, c->fft_err);
 }
 
 int fail(sbd_ctx* c, const Error& e) {
@@ -760,6 +791,9 @@ int sbd_create(sbd_ctx** out, int rows, int cols, int psf_size, int model, doubl
         SBD_REQUIRE(psf_size <= rows && psf_size <= cols, SBD_E_INVALID, "sbd_create: PSF larger than the image");
         SBD_REQUIRE(model >= 0 && model <= 2, SBD_E_INVALID, "sbd_create: unknown PSF model");
         SBD_REQUIRE(max_batch >= 1, SBD_E_INVALID, "sbd_create: max_batch must be >= 1");
+        // FFT size class from the size alone (no device needed).  A size the FFT operators refuse still makes a context:
+        // the TV entry points take any size >= 2; the FFT entry points then fail with this message.
+        const std::string fft_err = fft_size_error(rows, cols);
         int ndev = 0;
         cudaError_t e = cudaGetDeviceCount(&ndev);
         if (e != cudaSuccess || ndev == 0)
@@ -776,6 +810,8 @@ int sbd_create(sbd_ctx** out, int rows, int cols, int psf_size, int model, doubl
         c->max_batch = max_batch;
         c->npix = (size_t)rows * cols;
         c->pow2 = is_pow2(rows) && is_pow2(cols) && rows >= 16 && cols >= 16 && rows <= 4096 && cols <= 4096;
+        c->smooth = !c->pow2 && fft_err.empty();
+        c->fft_err = fft_err;
         c->nk = rows / 2 + 1;
         c->sp = 0;
         if (c->pow2) {
@@ -807,6 +843,11 @@ int sbd_create(sbd_ctx** out, int rows, int cols, int psf_size, int model, doubl
             c->cols_smem = (size_t)KC * le_y * 16;
         }
         c->spec_elems = (size_t)c->ntiles * cols * c->colsC;
+        if (c->smooth) {                // column-contiguous spec[img][k][q]
+            any_plan(rows, &c->plan_x);
+            any_plan(cols, &c->plan_y);
+            c->spec_elems = (size_t)c->nk * cols;
+        }
         {
             auto env_int = [](const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; };
             c->opt_chamb_seg = env_int("SBD_CHAMB_SEG", -1); c->opt_chamb_T = env_int("SBD_CHAMB_T", -1);
@@ -837,7 +878,7 @@ int sbd_create(sbd_ctx** out, int rows, int cols, int psf_size, int model, doubl
         c->ximg = dalloc<double>(c->npix);
         c->in_y = dalloc<double>(c->npix);          // staging image of the host-pointer entries (not allocated per call)
         SBD_CUDA(cudaMemsetAsync(c->ctl, 0, sizeof(Control), c->stream));
-        if (c->pow2) {
+        if (c->pow2 || c->smooth) {
             c->tw_nx = dalloc<double2>(rows); c->tw_ny = dalloc<double2>(cols);
             make_twiddles(rows, c->tw_nx, c->stream);
             make_twiddles(cols, c->tw_ny, c->stream);
@@ -900,7 +941,7 @@ int sbd_psf_spectrum(sbd_ctx* c, const double psi[2], int which, double* re, dou
     if (!c) return SBD_E_INVALID;
     SBD_TRY(c)
     SBD_REQUIRE(psi && re && im && which >= 0 && which <= 2, SBD_E_INVALID, "sbd_psf_spectrum: bad argument");
-    require_pow2(c);
+    require_fft(c);
     SBD_CUDA(cudaSetDevice(c->device));
     ensure_ws(c, 1);
     psf_from_host(c, psi, c->nx);
@@ -920,7 +961,7 @@ int sbd_blur_dev(sbd_ctx* c, const double* d_x, const double psi[2], int op, dou
     SBD_REQUIRE(d_x && d_out && psi && op >= 0 && op <= 3 && batch >= 1, SBD_E_INVALID, "sbd_blur: bad argument");
     SBD_REQUIRE(batch <= c->max_batch, SBD_E_INVALID, "sbd_blur: batch exceeds max_batch");
     SBD_REQUIRE(!(op == SBD_OP_D1 && c->model == SBD_LAPLACE), SBD_E_INVALID, "sbd_blur: Laplace PSF has one parameter");
-    require_pow2(c);
+    require_fft(c);
     SBD_CUDA(cudaSetDevice(c->device));
     ensure_ws(c, batch);
     psf_from_host(c, psi, c->nk);
@@ -1071,7 +1112,7 @@ int sbd_likelihood(sbd_ctx* c, const double* x, const double* y, const double ps
     if (!c) return SBD_E_INVALID;
     SBD_TRY(c)
     SBD_REQUIRE(x && y && psi && scal, SBD_E_INVALID, "sbd_likelihood: bad argument");
-    require_pow2(c);
+    require_fft(c);
     SBD_CUDA(cudaSetDevice(c->device));
     ensure_ws(c, 1);
     const size_t bytes = sizeof(double) * c->npix;
@@ -1117,11 +1158,11 @@ int sbd_max_eigenval(sbd_ctx* c, const double psi[2], const double* x0, double t
     if (!c) return SBD_E_INVALID;
     SBD_TRY(c)
     SBD_REQUIRE(psi && val && max_iter >= 1, SBD_E_INVALID, "sbd_max_eigenval: bad argument");
-    require_pow2(c);
+    require_fft(c);
     SBD_CUDA(cudaSetDevice(c->device));
     ensure_ws(c, 1);
     const size_t n = c->npix, bytes = sizeof(double) * n;
-    const unsigned gb = (unsigned)((n + 255) / 256), gp = (unsigned)((n / 2 + 255) / 256);
+    const unsigned gb = (unsigned)((n + 255) / 256), gp = (unsigned)(((n + 1) / 2 + 255) / 256);
     double* zero = c->ximg;                                         // all-zero image for the norms
     SBD_CUDA(cudaMemsetAsync(zero, 0, bytes, c->stream));
     if (x0) SBD_CUDA(cudaMemcpyAsync(c->X, x0, bytes, cudaMemcpyHostToDevice, c->stream));
@@ -1150,11 +1191,11 @@ int sbd_observe(sbd_ctx* c, const double* x, const double psi[2], double bsnr, c
     if (!c) return SBD_E_INVALID;
     SBD_TRY(c)
     SBD_REQUIRE(x && psi && y, SBD_E_INVALID, "sbd_observe: bad argument");
-    require_pow2(c);
+    require_fft(c);
     SBD_CUDA(cudaSetDevice(c->device));
     ensure_ws(c, 1);
     const size_t n = c->npix, bytes = sizeof(double) * n;
-    const unsigned gb = (unsigned)((n + 255) / 256), gp = (unsigned)((n / 2 + 255) / 256);
+    const unsigned gb = (unsigned)((n + 255) / 256), gp = (unsigned)(((n + 1) / 2 + 255) / 256);
     SBD_CUDA(cudaMemcpyAsync(c->X, x, bytes, cudaMemcpyHostToDevice, c->stream));
     psf_from_host(c, psi, c->nk);
     rows_fwd(c, c->X, c->S1, 1); cols<COL_OP>(c, c->S1, c->S1, 1, SBD_OP_A); rows_inv(c, c->S1, c->P, 1);        // Ax  :145
@@ -1190,7 +1231,7 @@ int sbd_salsa_tv(sbd_ctx* c, const double* y, const double psi[2], double tau, d
     int rc = SBD_OK;
     try {
         SBD_REQUIRE(y && psi && x && maxiter >= 1 && tv_iters >= 1 && mu > 0.0, SBD_E_INVALID, "sbd_salsa_tv: bad argument");
-        require_pow2(c);
+        require_fft(c);
         SBD_CUDA(cudaSetDevice(c->device));
         ensure_ws(c, 1);
         cudaStream_t s = c->stream;
@@ -1338,7 +1379,7 @@ void copy_trace(double* dst, const double* src, size_t n, cudaStream_t s) {
 
 void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const double* d_xtrue,
                    const sbd_params* prm, const double* d_noise, sbd_traces* out) {
-    require_pow2(c);
+    require_fft(c);
     SBD_REQUIRE(prm && out, SBD_E_INVALID, "sbd_sapg_run: params/traces NULL");
     const int nch = prm->n_chains;
     SBD_REQUIRE(nch >= 1 && nch <= c->max_batch, SBD_E_INVALID, "sbd_sapg_run: n_chains must be in [1, max_batch]");
@@ -1460,7 +1501,7 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     // are bit-identical to the serial order (SBD_OVERLAP=0 / sbd_set_option("overlap", 0); profiling runs serially).
     auto unit = [&](int mode, bool grad_after) {
         { PhaseTimer pt(c, 1);
-          const unsigned gx = (unsigned)((c->npix / 2 + 255) / 256);
+          const unsigned gx = (unsigned)(((c->npix + 1) / 2 + 255) / 256);
           k_langevin<<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->ctl, k.gam, k.lamb, k.sq2gam,
                                                    c->npix, nch, prm->seed, prm->chain_offset, burnIn);
           LAUNCH_CHECK(c);
