@@ -268,6 +268,29 @@ int sbd_phase_times(const sbd_ctx* ctx, double ms[SBD_N_PHASES], long long calls
 const char* sbd_phase_name(int i);
 
 /* ------------------------------------------------------------------------
+ * Posterior statistics of X (no reference counterpart: the reference stubs a
+ * Welford accumulator, SAPG_algorithm_Guassian.m:233-235,246,292-293).  For each
+ * chain c and block size s = 2^j, j = 0 .. L-1, Welford accumulators (m_c, M2_c)
+ * of the block mean over the samples X_ii, ii = burnIn+1 .. samples (the window
+ * of post_mean; n = samples - burnIn per chain).  Block (I,J) covers rows
+ * [I*s, min((I+1)*s, rows)) x cols [J*s, min((J+1)*s, cols)) and its mean divides
+ * by the pixels it actually holds.  Per block the device returns, over the C chains
+ * of this context in local chain order:
+ *   mean = (sum_c m_c) / C   (at s = 1 bitwise X_mean),  within = sum_c M2_c,
+ *   between = sum_c (m_c - mean)^2.
+ * From these: var = (within + n*between) / (C*n - 1), std = sqrt(var), and the
+ * Gelman-Rubin Rhat = sqrt(((n-1)/n * W + B/n) / W) with W = within / (C(n-1)),
+ * B/n = between / (C-1) (NaN for C < 2 or n < 2).  DESIGN.md "Posterior statistics".
+ * ---------------------------------------------------------------------- */
+/* 0 (default): off.  L in 1..7: every following sbd_sapg_run / sbd_sapg_run_dev accumulates the posterior moments of
+   X over ii = burnIn+1..samples at block sizes 1, 2, ..., 2^(L-1) (see DESIGN.md).  Requires burnIn >= 1. */
+int sbd_set_posterior(sbd_ctx* ctx, int levels);
+/* statistics of the last run at block size 2^level: mean, within, between are ceil(rows/s) x ceil(cols/s)
+   (each nullable); n = samples per chain, chains = C on this context. */
+int sbd_posterior_stats(const sbd_ctx* ctx, int level, double* mean, double* within, double* between,
+                        int* n, int* chains);
+
+/* ------------------------------------------------------------------------
  * Launch-geometry control (no reference counterpart: the reference has no
  * launch geometry).  Used by the parity tests to pin the production geometry
  * of the fused Chambolle kernel at sizes the oracle finishes quickly, and by

@@ -96,6 +96,8 @@ SIGNATURES = {
     "sbd_phase_times": (C.c_int, [C.c_void_p, c_double_p, C.POINTER(C.c_longlong)]),
     "sbd_set_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "sbd_phase_name": (C.c_char_p, [C.c_int]),
+    "sbd_set_posterior": (C.c_int, [C.c_void_p, C.c_int]),
+    "sbd_posterior_stats": (C.c_int, [C.c_void_p, C.c_int, c_double_p, c_double_p, c_double_p, c_int_p, c_int_p]),
     "sbd_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),
     "sbd_get_geometry": (C.c_int, [C.c_void_p, C.c_int, c_int_p]),
 }

@@ -18,9 +18,12 @@ namespace sbd {
 // grid = (ceil(ceil(npix/2)/blockDim), n_chains)
 // An odd npix puts the element pairs of every other chain off the 16-byte grid: scalar accesses there, and the last
 // element of an image (a pair of its own) takes z0 of its pair (oracle/philox.py).
+// M2: also accumulate the per-chain sum of squared deviations (Welford) next to the running mean; post_m2 is then
+// non-null whenever post_mean is.  The mean update is the same expression either way, so X_mean does not change.
+template <bool M2>
 __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
                            const double* __restrict__ Gf, const double* __restrict__ noise,
-                           double* __restrict__ post_mean, const Control* __restrict__ ctl,
+                           double* __restrict__ post_mean, double* __restrict__ post_m2, const Control* __restrict__ ctl,
                            double gam, double lamb, double sq2gam, size_t npix, int n_chains,
                            uint64_t seed, int chain_offset, int burnIn) {
     const size_t pair = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -45,7 +48,9 @@ __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
             X[off + e] = r;
             if (acc) {
                 const double inv = 1.0 / (double)(ctl->ii - burnIn);
-                post_mean[off + e] += (r - post_mean[off + e]) * inv;
+                const double m = post_mean[off + e], d = r - m, mn = m + d * inv;
+                post_mean[off + e] = mn;
+                if (M2) post_m2[off + e] += d * (r - mn);
             }
         }
         return;
@@ -69,9 +74,16 @@ __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
         // Guassian.m:233-235,246)
         const double inv = 1.0 / (double)(ctl->ii - burnIn);
         double2 m = *reinterpret_cast<double2*>(post_mean + off);
-        m.x += (r.x - m.x) * inv;
-        m.y += (r.y - m.y) * inv;
+        const double2 d = make_double2(r.x - m.x, r.y - m.y);
+        m.x += d.x * inv;
+        m.y += d.y * inv;
         *reinterpret_cast<double2*>(post_mean + off) = m;
+        if (M2) {   // M2 += d * (r - m_new)   (Welford; block sizes > 1: k_post_blocks)
+            double2 q = *reinterpret_cast<double2*>(post_m2 + off);
+            q.x += d.x * (r.x - m.x);
+            q.y += d.y * (r.y - m.y);
+            *reinterpret_cast<double2*>(post_m2 + off) = q;
+        }
     }
 }
 
@@ -238,6 +250,92 @@ __global__ void k_chain_mean(const double* __restrict__ in, double* __restrict__
     double s = 0.0;
     for (int c = 0; c < n; ++c) s += in[(size_t)c * npix + i];
     out[i] = s / (double)n;
+}
+
+// ---- posterior moments at block sizes s = 2^j (DESIGN.md "Posterior statistics") --------------------------------
+// Per chain and block, Welford accumulators over the main-loop samples ii = burnIn+1 .. samples of the block mean
+// v = (sum of the block) / (pixels it contains):  d = v - m;  m += d / n_ii;  M2 += d (v - m),  n_ii = ii - burnIn.
+// j = 0 is the pixel scale (k_langevin<true>); k_post_blocks does j = 1 .. levels-1.
+constexpr int POST_MAXL = 7;                // block sizes 1 .. 64
+constexpr int POST_TILE = 64;               // pixels per side of the tile one thread block reduces
+struct PostGeom {
+    int rows, cols, levels, tiles_x;        // tiles_x = ceil(rows / POST_TILE)
+    int bx[POST_MAXL], by[POST_MAXL];       // blocks along rows / cols at level j: ceil(rows / 2^j), ceil(cols / 2^j)
+    size_t off[POST_MAXL];                  // level j >= 1: offset of its [n_chains][bx*by] accumulators
+};
+
+__device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __restrict__ bm2, const PostGeom& g,
+                                             int j, int ch, int tx, int ty, int a, int b, double sum, double inv) {
+    const int n = POST_TILE >> j, I = tx * n + a, J = ty * n + b;
+    if (I >= g.bx[j] || J >= g.by[j]) return;
+    const int s = 1 << j;
+    const int cnt = (min((I + 1) * s, g.rows) - I * s) * (min((J + 1) * s, g.cols) - J * s);  // partial edge blocks
+    const double v = sum / (double)cnt;
+    const size_t idx = g.off[j] + (size_t)ch * g.bx[j] * g.by[j] + (size_t)J * g.bx[j] + I;
+    const double m = bm[idx], d = v - m, mn = m + d * inv;
+    bm[idx] = mn;
+    bm2[idx] += d * (v - mn);
+}
+
+// One 64 x 64 tile of one chain's new sample per block, grid = (tiles, n_chains).  Level 1 sums 2 x 2 pixels read
+// straight from X, every further level sums 2 x 2 sums of the level below in shared memory, always as
+// (top-left + bottom-left) + (top-right + bottom-right) with zeros outside the image: the order depends only on
+// rows, cols and the level.  Runs only in the main loop after burn-in (Control, so a captured graph stays valid).
+__global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ X, double* __restrict__ bm,
+                                                     double* __restrict__ bm2, const PostGeom g,
+                                                     const Control* __restrict__ ctl, int burnIn) {
+    __shared__ double sm[32 * 32 + 16 * 16 + 8 * 8 + 4 * 4 + 2 * 2 + 1];
+    if (!(ctl->phase == 1 && ctl->ii > burnIn)) return;
+    const double inv = 1.0 / (double)(ctl->ii - burnIn);
+    const int ch = blockIdx.y, tx = blockIdx.x % g.tiles_x, ty = blockIdx.x / g.tiles_x;
+    const int rows = g.rows, cols = g.cols;
+    const double* x = X + (size_t)ch * rows * cols;
+    for (int e = threadIdx.x; e < 32 * 32; e += blockDim.x) {
+        const int a = e & 31, b = e >> 5;
+        const int i = tx * POST_TILE + 2 * a, j = ty * POST_TILE + 2 * b;
+        const bool i0 = i < rows, i1 = i + 1 < rows, j0 = j < cols, j1 = j + 1 < cols;
+        const double* p = x + (size_t)j * rows + i;
+        const double v00 = (i0 && j0) ? p[0] : 0.0, v10 = (i1 && j0) ? p[1] : 0.0;
+        const double v01 = (i0 && j1) ? p[rows] : 0.0, v11 = (i1 && j1) ? p[rows + 1] : 0.0;
+        const double sum = (v00 + v10) + (v01 + v11);
+        sm[e] = sum;
+        post_welford(bm, bm2, g, 1, ch, tx, ty, a, b, sum, inv);
+    }
+    const double* prev = sm;
+    double* cur = sm + 32 * 32;
+#pragma unroll      // constant level indices: the PostGeom arrays stay in the parameter bank (no local copy)
+    for (int lv = 2; lv < POST_MAXL; ++lv) {
+        if (lv >= g.levels) break;
+        __syncthreads();
+        const int n = POST_TILE >> lv, n2 = 2 * n;
+        for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
+            const int a = e % n, b = e / n;
+            const double* q = prev + 2 * b * n2 + 2 * a;
+            const double sum = (q[0] + q[1]) + (q[n2] + q[n2 + 1]);
+            cur[e] = sum;
+            post_welford(bm, bm2, g, lv, ch, tx, ty, a, b, sum, inv);
+        }
+        prev = cur;
+        cur += n * n;
+    }
+}
+
+// Over the chains of this context, per element of one level (local chain order, as k_chain_mean):
+// mean = (sum_c m_c) / C,  within = sum_c M2_c,  between = sum_c (m_c - mean)^2
+__global__ void k_post_finalize(const double* __restrict__ m, const double* __restrict__ m2, size_t nb, int n,
+                                double* __restrict__ mean, double* __restrict__ within, double* __restrict__ between) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nb) return;
+    double s = 0.0;
+    for (int c = 0; c < n; ++c) s += m[(size_t)c * nb + i];
+    const double mu = s / (double)n;
+    double w = 0.0, b = 0.0;
+    for (int c = 0; c < n; ++c) {
+        w += m2[(size_t)c * nb + i];
+        const double d = m[(size_t)c * nb + i] - mu;
+        b += d * d;
+    }
+    mean[i] = mu; within[i] = w; between[i] = b;
 }
 
 // sum of x over one image -> out[0]   (mean(mean(Ax)), run_Gaussian_demo.m:148)

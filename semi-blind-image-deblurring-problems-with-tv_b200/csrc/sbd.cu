@@ -122,6 +122,13 @@ struct sbd_ctx {
     double *ximg = nullptr;         // 1-image staging (y, x_true)
     double *post = nullptr;
     int post_batch = 0;
+    // posterior statistics (sbd_set_posterior / sbd_posterior_stats, DESIGN.md "Posterior statistics")
+    int post_levels = 0;                    // sticky request: block sizes 1 .. 2^(post_levels-1), 0 = off
+    double* post_m2 = nullptr;              // pixel-scale M2 next to `post`, [post_m2_batch][npix]
+    int post_m2_batch = 0;
+    double* post_blk = nullptr; size_t post_blk_cap = 0;    // m and M2 of the levels >= 1, [2][sum_j n_chains*nb_j]
+    double* post_out = nullptr; size_t post_out_cap = 0;    // mean, within, between of every level of the last run
+    int stat_levels = 0, stat_n = 0, stat_chains = 0;       // what post_out holds (stat_levels 0: nothing)
 
     // per-run scratch kept across calls (a cudaMalloc / cudaFree per sbd_sapg_run costs up to 0.6 s: a free tears down
     // whatever the driver deferred, e.g. the graphs of the run)
@@ -708,6 +715,12 @@ void require_fft(sbd_ctx* c) {
     SBD_REQUIRE(c->pow2 || c->smooth, SBD_E_UNSUPPORTED, c->fft_err);
 }
 
+// elements of one image at block size 2^level: ceil(rows / s) x ceil(cols / s)
+size_t post_blocks(const sbd_ctx* c, int level) {
+    const int s = 1 << level;
+    return (size_t)((c->nx + s - 1) / s) * (size_t)((c->ny + s - 1) / s);
+}
+
 int fail(sbd_ctx* c, const Error& e) {
     if (c) c->err = e.msg; else g_create_error = e.msg;
     return e.code;
@@ -747,6 +760,40 @@ int sbd_set_profile(sbd_ctx* ctx, int on) {
     if (!ctx) return SBD_E_INVALID;
     ctx->profile = on != 0;
     return SBD_OK;
+}
+
+int sbd_set_posterior(sbd_ctx* c, int levels) {
+    if (!c) return SBD_E_INVALID;
+    if (levels < 0 || levels > POST_MAXL) {
+        c->err = "sbd_set_posterior: levels must be in 0..7 (block sizes 1 .. 2^(levels-1))";
+        return SBD_E_INVALID;
+    }
+    c->post_levels = levels;
+    return SBD_OK;
+}
+
+int sbd_posterior_stats(const sbd_ctx* ctx, int level, double* mean, double* within, double* between, int* n,
+                        int* chains) {
+    if (!ctx) return SBD_E_INVALID;
+    sbd_ctx* c = const_cast<sbd_ctx*>(ctx);     // only the error text and the stream are touched
+    SBD_TRY(c)
+    SBD_REQUIRE(c->stat_levels > 0, SBD_E_INVALID,
+                "sbd_posterior_stats: the last SAPG run on this context accumulated no statistics (sbd_set_posterior)");
+    SBD_REQUIRE(level >= 0 && level < c->stat_levels, SBD_E_INVALID,
+                "sbd_posterior_stats: level " + std::to_string(level) + " outside 0.." + std::to_string(c->stat_levels - 1) +
+                " of the last run");
+    SBD_CUDA(cudaSetDevice(c->device));
+    size_t off = 0;
+    for (int j = 0; j < level; ++j) off += 3 * post_blocks(c, j);
+    const size_t nb = post_blocks(c, level);
+    double* dst[3] = {mean, within, between};
+    for (int q = 0; q < 3; ++q)
+        if (dst[q]) SBD_CUDA(cudaMemcpyAsync(dst[q], c->post_out + off + q * nb, nb * sizeof(double), cudaMemcpyDeviceToHost,
+                                             c->stream));
+    SBD_CUDA(cudaStreamSynchronize(c->stream));
+    if (n) *n = c->stat_n;
+    if (chains) *chains = c->stat_chains;
+    SBD_CATCH(c)
 }
 
 int sbd_set_option(sbd_ctx* c, const char* name, int value) {
@@ -904,6 +951,7 @@ int sbd_destroy(sbd_ctx* c) {
     dfree(c->in_y); dfree(c->in_x0); dfree(c->in_xt);
     dfree(c->tw_nx); dfree(c->tw_ny); dfree(c->taps); dfree(c->coef); dfree(c->ctl); dfree(c->psi_dev);
     dfree(c->ximg); dfree(c->yhat); dfree(c->allstats); dfree(c->post);
+    dfree(c->post_m2); dfree(c->post_blk); dfree(c->post_out);
     dfree(c->trace_d); dfree(c->trace_i); dfree(c->sal_aty); dfree(c->sal_u); dfree(c->sal_bu); dfree(c->sal_xt);
     if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
     if (c->ev_langevin) cudaEventDestroy(c->ev_langevin);
@@ -1385,6 +1433,9 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     SBD_REQUIRE(nch >= 1 && nch <= c->max_batch, SBD_E_INVALID, "sbd_sapg_run: n_chains must be in [1, max_batch]");
     SBD_REQUIRE(prm->samples >= 1 && prm->warmup >= 0, SBD_E_INVALID, "sbd_sapg_run: samples >= 1, warmup >= 0");
     SBD_REQUIRE(prm->chambolle_maxiter >= 1, SBD_E_INVALID, "sbd_sapg_run: chambolle_maxiter >= 1");
+    c->stat_levels = 0;
+    SBD_REQUIRE(c->post_levels == 0 || prm->burnIn >= 1, SBD_E_INVALID,
+                "sbd_sapg_run: posterior statistics (sbd_set_posterior) need burnIn >= 1");
     const int ntot = std::max(prm->total_chains, nch);
     if (c->comm) SBD_REQUIRE(ntot == nch * c->nranks, SBD_E_INVALID, "sbd_sapg_run: total_chains must be n_chains * nranks");
     else SBD_REQUIRE(ntot == nch, SBD_E_COMM, "sbd_sapg_run: total_chains > n_chains needs sbd_comm_init");
@@ -1438,11 +1489,34 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
         dt.t.delta = dt.delta;
     }
     if (ntot > c->allstats_cap) { dfree(c->allstats); c->allstats = dalloc<double>((size_t)ntot * NSTAT); c->allstats_cap = ntot; }
+    // posterior statistics: the running mean becomes required, M2 sits next to it; blocks of size >= 2 in post_blk
+    const int L = c->post_levels;
     double* post = nullptr;
-    if (prm->post_mean) {
+    if (prm->post_mean || L > 0) {
         if (c->post_batch < nch) { dfree(c->post); c->post = dalloc<double>((size_t)nch * c->npix); c->post_batch = nch; }
         post = c->post;
         SBD_CUDA(cudaMemsetAsync(post, 0, sizeof(double) * nch * c->npix, s));
+    }
+    PostGeom pg;
+    memset(&pg, 0, sizeof pg);
+    size_t blk_half = 0, out_elems = 0;
+    unsigned post_tiles = 0;
+    if (L > 0) {
+        if (c->post_m2_batch < nch) {
+            dfree(c->post_m2); c->post_m2 = dalloc<double>((size_t)nch * c->npix); c->post_m2_batch = nch;
+        }
+        SBD_CUDA(cudaMemsetAsync(c->post_m2, 0, sizeof(double) * nch * c->npix, s));
+        pg.rows = c->nx; pg.cols = c->ny; pg.levels = L; pg.tiles_x = (c->nx + POST_TILE - 1) / POST_TILE;
+        for (int j = 0; j < L; ++j) {
+            const int sz = 1 << j;
+            pg.bx[j] = (c->nx + sz - 1) / sz; pg.by[j] = (c->ny + sz - 1) / sz;
+            if (j >= 1) { pg.off[j] = blk_half; blk_half += (size_t)nch * post_blocks(c, j); }
+            out_elems += 3 * post_blocks(c, j);
+        }
+        post_tiles = (unsigned)(pg.tiles_x * ((c->ny + POST_TILE - 1) / POST_TILE));
+        if (2 * blk_half > c->post_blk_cap) { dfree(c->post_blk); c->post_blk = dalloc<double>(2 * blk_half); c->post_blk_cap = 2 * blk_half; }
+        if (out_elems > c->post_out_cap) { dfree(c->post_out); c->post_out = dalloc<double>(out_elems); c->post_out_cap = out_elems; }
+        if (blk_half) SBD_CUDA(cudaMemsetAsync(c->post_blk, 0, sizeof(double) * 2 * blk_half, s));
     }
 
     cudaEvent_t ev0, ev1;
@@ -1502,8 +1576,14 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     auto unit = [&](int mode, bool grad_after) {
         { PhaseTimer pt(c, 1);
           const unsigned gx = (unsigned)(((c->npix + 1) / 2 + 255) / 256);
-          k_langevin<<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->ctl, k.gam, k.lamb, k.sq2gam,
-                                                   c->npix, nch, prm->seed, prm->chain_offset, burnIn);
+          if (L > 0)
+              k_langevin<true><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->post_m2, c->ctl, k.gam,
+                                                             k.lamb, k.sq2gam, c->npix, nch, prm->seed, prm->chain_offset,
+                                                             burnIn);
+          else
+              k_langevin<false><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, nullptr, c->ctl, k.gam,
+                                                              k.lamb, k.sq2gam, c->npix, nch, prm->seed, prm->chain_offset,
+                                                              burnIn);
           LAUNCH_CHECK(c);
           if (mark_langevin) SBD_CUDA(cudaEventRecord(c->ev_langevin, s)); }
         const bool ov = c->opt_overlap != 0 && !c->profile;
@@ -1519,6 +1599,11 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
             }
         } else {
             prox(mode);
+        }
+        if (L >= 2 && mode == 2) {      // block moments of the new sample; reads X, like the prox next to it
+            PhaseTimer pt(c, 1);
+            k_post_blocks<<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, pg, c->ctl, burnIn);
+            LAUNCH_CHECK(c);
         }
         analyse(c, nch);
         if (d_xtrue) {
@@ -1639,10 +1724,22 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
         SBD_CUDA(cudaMemcpyAsync(out->chambolle_iters, dt.t.chamb_k, sizeof(int) * samples, cudaMemcpyDeviceToHost, s));
     if (out->X_last && !overlap_xlast)
         SBD_CUDA(cudaMemcpyAsync(out->X_last, c->X, sizeof(double) * nch * c->npix, cudaMemcpyDeviceToHost, s));
-    if (out->X_mean && post) {
+    if (out->X_mean && prm->post_mean) {
         k_chain_mean<<<(unsigned)((c->npix + 255) / 256), 256, 0, s>>>(post, c->Gf, c->npix, nch);
         LAUNCH_CHECK(c);
         SBD_CUDA(cudaMemcpyAsync(out->X_mean, c->Gf, sizeof(double) * c->npix, cudaMemcpyDeviceToHost, s));
+    }
+    {   // posterior statistics over this context's chains, per level (sbd_posterior_stats copies them out)
+        size_t off = 0;
+        for (int j = 0; j < L; ++j) {
+            const size_t nb = post_blocks(c, j);
+            const double* m = j == 0 ? post : c->post_blk + pg.off[j];
+            const double* m2 = j == 0 ? c->post_m2 : c->post_blk + blk_half + pg.off[j];
+            k_post_finalize<<<(unsigned)((nb + 255) / 256), 256, 0, s>>>(m, m2, nb, nch, c->post_out + off,
+                                                                        c->post_out + off + nb, c->post_out + off + 2 * nb);
+            LAUNCH_CHECK(c);
+            off += 3 * nb;
+        }
     }
     SBD_CUDA(cudaStreamSynchronize(s));
     if (overlap_xlast) SBD_CUDA(cudaStreamSynchronize(c->copy_stream));
@@ -1656,6 +1753,7 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     c->profile = want_profile;
     resolve_phase_events(c);
     out->last_samp = samples;                                       // Guassian.m:252 (no early break, Q10)
+    if (L > 0) { c->stat_levels = L; c->stat_n = std::max(samples - burnIn, 0); c->stat_chains = nch; }
 
     // ---- host post-processing of the scalar trajectories (Guassian.m:218-247,258-284)
     if (out->thetas) memcpy(out->thetas, th.data(), sizeof(double) * samples);

@@ -32,6 +32,27 @@ def _psi(psi):
     return v
 
 
+def posterior_moments(mean, within, between, n, chains):
+    """var, std and Gelman-Rubin Rhat from the sufficient statistics sbd_posterior_stats returns (DESIGN.md
+    "Posterior statistics"): n samples per chain, `chains` chains.
+      var  = (within + n*between) / (C*n - 1)                     (NaN for C*n < 2)
+      W    = within / (C(n-1)),  B/n = between / (C-1),  V = (n-1)/n * W + B/n,  Rhat = sqrt(V / W)
+                                                                  (NaN for C < 2 or n < 2)"""
+    within = np.asarray(within, dtype=np.float64)
+    between = np.asarray(between, dtype=np.float64)
+    n, C_ = int(n), int(chains)
+    nan = np.full(within.shape, np.nan)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        var = (within + n * between) / (C_ * n - 1) if C_ * n >= 2 else nan.copy()
+        if C_ >= 2 and n >= 2:
+            W = within / (C_ * (n - 1))
+            V = (n - 1) / n * W + between / (C_ - 1)
+            rhat = np.sqrt(V / W)
+        else:
+            rhat = nan.copy()
+    return var, np.sqrt(var), rhat
+
+
 class Engine:
     """One libsbd context: fixed image size, PSF family and GPU."""
 
@@ -202,9 +223,28 @@ class Engine:
                     mses=mses[:k + 1] if x_true is not None else np.zeros(0), n_outer=k, numA=k + 1, numAt=1)
 
     # -- SAPG -----------------------------------------------------------------
-    def sapg(self, y, prm, X0=None, x_true=None, noise=None, want_X_warm=True, want_X_mean=False):
+    def set_posterior(self, levels):
+        """sbd_set_posterior: 0 off, L in 1..7 accumulates posterior moments at block sizes 1 .. 2^(L-1) in every
+        following run (sticky on the context)."""
+        self._check(lib.sbd_set_posterior(self._h, int(levels)))
+
+    def posterior_stats(self, level):
+        """Statistics of the last run at block size 2^level: dict(scale, n, chains, mean, within, between, var, std,
+        Rhat), images ceil(rows/s) x ceil(cols/s)."""
+        s = 1 << int(level)
+        bx, by = -(-self.rows // s), -(-self.cols // s)
+        bufs = [np.zeros(bx * by) for _ in range(3)]
+        n, ch = C.c_int(), C.c_int()
+        self._check(lib.sbd_posterior_stats(self._h, int(level), *[_p(b) for b in bufs], C.byref(n), C.byref(ch)))
+        mean, within, between = (b.reshape(by, bx).T.copy() for b in bufs)
+        var, std, rhat = posterior_moments(mean, within, between, n.value, ch.value)
+        return dict(scale=s, n=n.value, chains=ch.value, mean=mean, within=within, between=between, var=var, std=std,
+                    Rhat=rhat)
+
+    def sapg(self, y, prm, X0=None, x_true=None, noise=None, want_X_warm=True, want_X_mean=False, post_levels=0):
         """Run sbd_sapg_run.  `prm` is a filled sbd_params; noise (optional)
-        is [(warmup-1)+(samples-1), n_chains, rows, cols]."""
+        is [(warmup-1)+(samples-1), n_chains, rows, cols].  post_levels L > 0 adds out["posterior"]: one
+        `posterior_stats` dict per block size 1 .. 2^(L-1); the context is left with the statistics off."""
         yb, _ = self._img(y, "y")
         x0b = self._img(X0, "X0")[0] if X0 is not None else None
         xtb = self._img(x_true, "x_true")[0] if x_true is not None else None
@@ -236,8 +276,16 @@ class Engine:
             xw = np.zeros(nch * self.rows * self.cols); tr.X_warm = _p(xw)
         if want_X_mean:
             xm = np.zeros(self.rows * self.cols); tr.X_mean = _p(xm)
-        self._check(lib.sbd_sapg_run(self._h, _p(yb), _p(x0b), _p(xtb), C.byref(prm), _p(nb), C.byref(tr)))
+        self.set_posterior(post_levels)
+        try:
+            self._check(lib.sbd_sapg_run(self._h, _p(yb), _p(x0b), _p(xtb), C.byref(prm), _p(nb), C.byref(tr)))
+            posterior = [self.posterior_stats(j) for j in range(int(post_levels))]
+        finally:
+            if post_levels:
+                lib.sbd_set_posterior(self._h, 0)
         out = dict(bufs)
+        if post_levels:
+            out["posterior"] = posterior
         out["logPiTrace_WU"] = bufs["logPiTrace_WU"][:W]
         for name in ("mean_theta", "mean_psi0", "mean_psi1", "mean_sigma"):
             out[name] = bufs[name][:nm]
@@ -465,7 +513,7 @@ def make_params(model, op, c=None, n_chains=1, seed=1, chain_offset=0, total_cha
     return p
 
 
-def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, x_true=None):
+def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, x_true=None, post_levels=0):
     y = np.asarray(y, dtype=np.float64)
     op = dict(op)
     if "warmup" not in op:
@@ -473,16 +521,26 @@ def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean
     prm = make_params(model, op, c, n_chains=n_chains, seed=seed, post_mean=post_mean)
     eng = engine or engine_for(y.shape, op["psf_size"], model, op.get("phi", 0.0), max_batch=n_chains)
     X0 = op.get("X0")                                                           # Guassian.m:10-12
-    out = eng.sapg(y, prm, X0=X0, x_true=x_true, noise=noise, want_X_mean=post_mean)
+    out = eng.sapg(y, prm, X0=X0, x_true=x_true, noise=noise, want_X_mean=post_mean, post_levels=post_levels)
     return op, prm, out
 
 
-def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False):
+def _add_posterior(r, o):
+    """results.posterior (one dict per block size) and, at the pixel scale, posteriorvar / posteriorstd / Rhat -
+    only when the statistics were requested, so that the default results keep the reference's field set."""
+    if "posterior" in o:
+        p0 = o["posterior"][0]
+        r.update(posterior=o["posterior"], posteriorvar=p0["var"], posteriorstd=p0["std"], Rhat=p0["Rhat"])
+    return r
+
+
+def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
     """[theta_EB, w1_EB, w2_EB, sigma_EB, results] = SAPG_algorithm_Guassian(y, op, c)
     SAPG/SAPG_algorithm_Guassian.m:7-308.  `op` must carry the plain-data fields
     the reference already stores (psf_size, phi, lambda, gamma, ...); the function
-    handles in `op` are not used - the engine implements the model they encode."""
-    op, prm, o = _run(GAUSSIAN, y, op, c, noise, n_chains, seed, engine, post_mean)
+    handles in `op` are not used - the engine implements the model they encode.  post_levels > 0 adds the posterior
+    statistics (Engine.sapg) as results["posterior"], ["posteriorvar"], ["posteriorstd"], ["Rhat"]."""
+    op, prm, o = _run(GAUSSIAN, y, op, c, noise, n_chains, seed, engine, post_mean, post_levels=post_levels)
     r = dict(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindParameters=o["seconds"], last_samp=o["last_samp"],
              logPiTraceX=o["logPiTraceX"], gXTrace=o["gXTrace"],
              theta_EB=o["EB"][0], last_theta=o["thetas"][-1], thetas=o["thetas"], mean_thetas=o["mean_theta"],
@@ -495,13 +553,14 @@ def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=Non
              grad_theta=o["grad_theta"], grad_w1=o["grad_psi0"], grad_w2=o["grad_psi1"],
              grad_sigma=o["grad_sigma"], options=op,
              chambolle_iters=o["chambolle_iters"], X_warm=o.get("X_warm"), posteriormean=o.get("X_mean"))
+    _add_posterior(r, o)
     return r["theta_EB"], r["w1_EB"], r["w2_EB"], r["sigma_EB"], r
 
 
-def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False):
+def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
     """[theta_EB, alpha_EB, beta_EB, sigma2_EB, results] = SAPG_algorithm_moffat(y, op)
     SAPG/SAPG_algorithm_moffat.m:7-297."""
-    op, prm, o = _run(MOFFAT, y, op, None, noise, n_chains, seed, engine, post_mean)
+    op, prm, o = _run(MOFFAT, y, op, None, noise, n_chains, seed, engine, post_mean, post_levels=post_levels)
     err_psf = o["err_psf"].copy(); err_psf[0] = 0.0          # err_psf(1) is never assigned (moffat.m:205)
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],
@@ -517,15 +576,17 @@ def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, po
              Xlast_sample=o["X_last"][0] if n_chains == 1 else o["X_last"],
              X_warm=o["X_warm"][0] if n_chains == 1 else o["X_warm"], options=op, err_psf=err_psf,
              chambolle_iters=o["chambolle_iters"], posteriormean=o.get("X_mean"))
+    _add_posterior(r, o)
     return r["mean_theta"], r["alpha_EB"], r["beta_EB"], r["sigma_EB"], r
 
 
-def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False):
+def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
     """[theta_EB, b_EB, sigma_EB, results] = SAPG_algorithm_laplace(y, op)
     SAPG/SAPG_algorithm_laplace.m:7-268 (needs op.x, the ground truth, :28)."""
     if "x" not in op:
         raise KeyError("Reference to non-existent field 'x'.")                 # laplace.m:28
-    op, prm, o = _run(LAPLACE, y, op, None, noise, n_chains, seed, engine, post_mean, x_true=op["x"])
+    op, prm, o = _run(LAPLACE, y, op, None, noise, n_chains, seed, engine, post_mean, x_true=op["x"],
+                      post_levels=post_levels)
     err_warm = np.zeros(max(int(op["warmup"]), 1)); err_warm[0] = o["err_warm0"]    # laplace.m:28-29
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],
@@ -540,4 +601,5 @@ def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, p
              X_warm=o["X_warm"][0] if n_chains == 1 else o["X_warm"],
              err_warm=err_warm, err_sample=o["err_sample"], err_psf=o["err_psf"], options=op,
              chambolle_iters=o["chambolle_iters"], posteriormean=o.get("X_mean"))
+    _add_posterior(r, o)
     return r["mean_theta"], r["mean_b"], r["sigma_EB"], r

@@ -22,4 +22,5 @@ results.c_theta = c.theta; results.c_w1 = c.w1; results.c_w2 = c.w2; results.Xla
 results.c_sigma = c.sigma; results.err_psf = r.err_psf;
 results.grad_theta = r.grad_theta; results.grad_w1 = r.grad_psi0; results.grad_w2 = r.grad_psi1;
 results.grad_sigma = r.grad_sigma; results.options = op;
+if isfield(r, 'posterior'), results = sbd_posterior(results, r); end   % only with op.post_levels > 0
 end

@@ -18,4 +18,5 @@ results.mean_sigmas = r.mean_sigma; results.tol_sigma = r.tol_sigma; results.c_s
 results.X_sample = r.X_last; results.X_warm = r.X_warm;
 results.err_warm = zeros(1, max(op.warmup, 1)); results.err_warm(1) = r.err_warm0;   % laplace.m:28-29
 results.err_sample = r.err_sample; results.err_psf = r.err_psf; results.options = op;
+if isfield(r, 'posterior'), results = sbd_posterior(results, r); end   % only with op.post_levels > 0
 end

@@ -18,4 +18,5 @@ results.sigma_EB = sigma2_EB; results.last_sigma = r.sigmas(end); results.sigmas
 results.mean_sigmas = r.mean_sigma; results.tol_sigma = r.tol_sigma; results.c_sigma2 = 10000;
 results.Xlast_sample = r.X_last; results.X_warm = r.X_warm; results.options = op;
 results.err_psf = r.err_psf; results.err_psf(1) = 0;          % err_psf(1) is never assigned (moffat.m:205)
+if isfield(r, 'posterior'), results = sbd_posterior(results, r); end   % only with op.post_levels > 0
 end

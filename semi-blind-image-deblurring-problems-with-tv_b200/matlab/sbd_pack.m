@@ -50,5 +50,6 @@ P.d_scale = op.d_scale; P.d_exp = op.d_exp; P.seed = 1;
 if isfield(op, 'seed'), P.seed = op.seed; end
 P.use_graph = -1;                                                    % automatic: CUDA-graph replay for small images
 if isfield(op, 'use_graph'), P.use_graph = op.use_graph; end
+if isfield(op, 'post_levels'), P.post_levels = op.post_levels; end   % posterior statistics (sbd_posterior.m)
 r2res = names;
 end

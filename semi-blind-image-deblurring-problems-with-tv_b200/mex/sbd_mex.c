@@ -19,6 +19,9 @@
  *   out     = sbd_mex('blur', x, model, t, phi, psi, op)                  A / AT / dif_* closures
  *   s       = sbd_mex('likelihood', x, y, model, t, phi, psi, sigma2, theta)   op.f, op.gradF, op.grad_psi, ...
  *   r       = sbd_mex('sapg', y, X0, xtrue, model, t, phi, P, noise)      SAPG/SAPG_algorithm_*.m
+ *             P.post_levels = L (optional, 0 = off) adds r.posterior: a 1x1 struct with one field per block size,
+ *             s1, s2, s4, ..., each a struct with scale, n, chains, mean, within, between, var, std, Rhat
+ *             (include/sbd.h sbd_posterior_stats; the .m wrappers turn it into a struct array)
  *   [v,k]   = sbd_mex('max_eigenval', [M N], model, t, phi, psi, tol, maxit, x0)   utils/max_eigenval_*.m
  *   [y,s,n] = sbd_mex('observe', x, model, t, phi, psi, bsnr, noise)      run_Gaussian_demo.m:145-168
  *   [x,obj,dist,mses] = sbd_mex('salsa', y, model, t, phi, psi, tau, mu, maxiter, tolA, tviters, xtrue)
@@ -27,6 +30,7 @@
  * Build:  mex -I../../include sbd_mex.c -L../lib -lsbd          (MATLAB)
  *         mkoctfile --mex -I../../include sbd_mex.c -L../lib -lsbd   (Octave)
  */
+#include <math.h>
 #include <string.h>
 #include <stdio.h>
 #include "mex.h"
@@ -98,6 +102,43 @@ static mxArray* vec(int n, double** p) {
     mxArray* a = mxCreateDoubleMatrix(1, n > 0 ? n : 0, mxREAL);
     *p = mxGetPr(a);
     return a;
+}
+
+/* posterior statistics of the last run at block sizes 1 .. 2^(levels-1), with var, std and Rhat formed as DESIGN.md
+   states them ("Posterior statistics") */
+static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels) {
+    static const char* fields[] = {"scale", "n", "chains", "mean", "within", "between", "var", "std", "Rhat"};
+    char lnames[8][8];
+    const char* lp[8];
+    mxArray* out;
+    int j, rc;
+    for (j = 0; j < levels; ++j) { snprintf(lnames[j], sizeof lnames[j], "s%d", 1 << j); lp[j] = lnames[j]; }
+    out = mxCreateStructMatrix(1, 1, levels, lp);
+    for (j = 0; j < levels; ++j) {
+        const int s = 1 << j, bx = (rows + s - 1) / s, by = (cols + s - 1) / s;
+        mxArray* e = mxCreateStructMatrix(1, 1, 9, fields);
+        mxArray *a[6];
+        double* p[6];
+        int q, n = 0, C = 0;
+        size_t i;
+        for (q = 0; q < 6; ++q) { a[q] = mxCreateDoubleMatrix(bx, by, mxREAL); p[q] = mxGetPr(a[q]); }
+        rc = sbd_posterior_stats(c, j, p[0], p[1], p[2], &n, &C);
+        if (rc) { sbd_set_posterior(c, 0); fail(c, "sbd_posterior_stats", rc); }
+        for (i = 0; i < (size_t)bx * by; ++i) {
+            const double W = p[1][i], B = p[2][i];
+            p[3][i] = C * n >= 2 ? (W + n * B) / (double)(C * n - 1) : NAN;            /* var */
+            p[4][i] = sqrt(p[3][i]);                                                 /* std */
+            p[5][i] = (C >= 2 && n >= 2)                                             /* Gelman-Rubin Rhat */
+                ? sqrt(((n - 1.0) / n * (W / (C * (n - 1.0))) + B / (C - 1.0)) / (W / (C * (n - 1.0)))) : NAN;
+        }
+        mxSetField(e, 0, "scale", mxCreateDoubleScalar((double)s));
+        mxSetField(e, 0, "n", mxCreateDoubleScalar((double)n));
+        mxSetField(e, 0, "chains", mxCreateDoubleScalar((double)C));
+        mxSetField(e, 0, "mean", a[0]); mxSetField(e, 0, "within", a[1]); mxSetField(e, 0, "between", a[2]);
+        mxSetField(e, 0, "var", a[3]); mxSetField(e, 0, "std", a[4]); mxSetField(e, 0, "Rhat", a[5]);
+        mxSetField(out, 0, lp[j], e);
+    }
+    return out;
 }
 
 void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
@@ -182,7 +223,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                                       "grad_psi1", "grad_sigma", "logPiTraceX", "gXTrace", "err_psf", "err_sample",
                                       "tol_theta", "tol_psi0", "tol_psi1", "tol_sigma", "mean_theta", "mean_psi0",
                                       "mean_psi1", "mean_sigma", "X_warm", "X_last", "EB", "err_warm0", "seconds",
-                                      "last_samp"};
+                                      "last_samp", "posterior"};
         const double* y = image(prhs[1], "y", &rows, &cols);
         const double* X0 = mxIsEmpty(prhs[2]) ? NULL : mxGetPr(prhs[2]);
         const double* xt = mxIsEmpty(prhs[3]) ? NULL : mxGetPr(prhs[3]);
@@ -192,7 +233,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         sbd_traces t;
         sbd_ctx* c;
         double* q[21];
-        int i, nm;
+        int i, nm, levels;
         mxArray* r;
         if (!mxIsStruct(P)) mexErrMsgIdAndTxt("sbd:type", "P must be a struct");
         memset(&p, 0, sizeof p); memset(&t, 0, sizeof t);
@@ -213,9 +254,11 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         p.d_scale = field(P, "d_scale", 1, 0); p.d_exp = field(P, "d_exp", 1, 0);
         p.seed = (uint64_t)field(P, "seed", 0, 1); p.chain_offset = 0; p.total_chains = p.n_chains;
         p.use_graph = (int)field(P, "use_graph", 0, -1);            /* -1: automatic (CUDA graph for small problems) */
+        levels = (int)field(P, "post_levels", 0, 0);                 /* posterior statistics, 0 = off */
         c = get_ctx(rows, cols, (int)mxGetScalar(prhs[5]), (int)mxGetScalar(prhs[4]), mxGetScalar(prhs[6]), p.n_chains);
         nm = p.samples - p.burnIn; if (nm < 0) nm = 0;
-        r = mxCreateStructMatrix(1, 1, (int)(sizeof names / sizeof names[0]), names);
+        /* the `posterior` field exists only when it was asked for: otherwise the old field set */
+        r = mxCreateStructMatrix(1, 1, (int)(sizeof names / sizeof names[0]) - (levels > 0 ? 0 : 1), names);
         for (i = 0; i < 21; ++i) {
             const int len = (i == 0) ? p.warmup : (i >= 17 ? nm : p.samples);
             mxSetField(r, 0, names[i], vec(len, &q[i]));
@@ -227,8 +270,15 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         t.mean_theta = q[17]; t.mean_psi0 = q[18]; t.mean_psi1 = q[19]; t.mean_sigma = q[20];
         { mxArray* a = mxCreateDoubleMatrix(rows, cols * p.n_chains, mxREAL); t.X_warm = mxGetPr(a); mxSetField(r, 0, "X_warm", a); }
         { mxArray* a = mxCreateDoubleMatrix(rows, cols * p.n_chains, mxREAL); t.X_last = mxGetPr(a); mxSetField(r, 0, "X_last", a); }
+        if ((rc = sbd_set_posterior(c, levels))) fail(c, "sbd_set_posterior", rc);
         rc = sbd_sapg_run(c, y, X0, xt, &p, noise, &t);
-        if (rc) fail(c, "sbd_sapg_run", rc);
+        if (rc) { sbd_set_posterior(c, 0); fail(c, "sbd_sapg_run", rc); }
+        if (levels > 0) {
+            mxArray* post;
+            post = posterior_struct(c, rows, cols, levels);
+            sbd_set_posterior(c, 0);                             /* cached context: the request is sticky */
+            mxSetField(r, 0, "posterior", post);
+        }
         { double* e; mxSetField(r, 0, "EB", vec(4, &e)); for (i = 0; i < 4; ++i) e[i] = t.EB[i]; }
         mxSetField(r, 0, "err_warm0", mxCreateDoubleScalar(t.err_warm0));
         mxSetField(r, 0, "seconds", mxCreateDoubleScalar(t.seconds));

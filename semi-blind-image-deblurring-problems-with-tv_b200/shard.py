@@ -75,3 +75,48 @@ class ChainShard:
         for ch in range(allv.shape[0]):          # fixed order
             tot = tot + allv[ch]
         return tot
+
+    def combine_posterior(self, stats):
+        """Merge the posterior statistics of every rank's chains (Engine.sapg(..., post_levels=L)["posterior"]: one
+        dict per block size with scale, n, chains, mean, within, between) into those of all chains.  Each rank's
+        (C_r, mean_r, within_r, between_r) is all-gathered and merged in rank order:
+            mean = sum_r C_r mean_r / C,  within = sum_r within_r,  between = sum_r [between_r + C_r (mean_r - mean)^2]
+        This is exact algebra, but it sums in another order than one context running all C chains, so the result
+        equals a one-GPU run to rounding (~1e-13 relative), not bit for bit.  Returns the same list of dicts with
+        var, std and Rhat recomputed from the merged statistics."""
+        from .host import posterior_moments
+        out = []
+        for st in stats:
+            mean = np.asarray(st["mean"], dtype=np.float64)
+            local = np.stack([mean, np.asarray(st["within"], dtype=np.float64),
+                              np.asarray(st["between"], dtype=np.float64)])
+            if self.world_size == 1:
+                parts, counts, ns = [local], [int(st["chains"])], [int(st["n"])]
+            else:
+                import torch
+                import torch.distributed as dist
+                mine = torch.from_numpy(np.ascontiguousarray(local))
+                gathered = [torch.empty_like(mine) for _ in range(self.world_size)]
+                dist.all_gather(gathered, mine)
+                meta = torch.tensor([int(st["chains"]), int(st["n"])], dtype=torch.int64)
+                metas = [torch.empty_like(meta) for _ in range(self.world_size)]
+                dist.all_gather(metas, meta)
+                parts = [g.numpy() for g in gathered]
+                counts = [int(m[0]) for m in metas]
+                ns = [int(m[1]) for m in metas]
+            if len(set(ns)) != 1:
+                raise ValueError(f"combine_posterior: ranks differ in samples per chain {ns}")
+            C_ = sum(counts)
+            tot = np.zeros_like(mean)
+            for cr, pr in zip(counts, parts):              # rank order
+                tot = tot + cr * pr[0]
+            m = tot / C_
+            within = np.zeros_like(mean)
+            between = np.zeros_like(mean)
+            for cr, pr in zip(counts, parts):
+                within = within + pr[1]
+                between = between + (pr[2] + cr * (pr[0] - m) ** 2)
+            var, std, rhat = posterior_moments(m, within, between, ns[0], C_)
+            out.append(dict(scale=st["scale"], n=ns[0], chains=C_, mean=m, within=within, between=between, var=var,
+                            std=std, Rhat=rhat))
+        return out
