@@ -291,6 +291,31 @@ int sbd_posterior_stats(const sbd_ctx* ctx, int level, double* mean, double* wit
                         int* n, int* chains);
 
 /* ------------------------------------------------------------------------
+ * Precision and convergence of the posterior statistics (no reference counterpart).  Over the same window and block
+ * sizes, per chain c and element:
+ *   batch means: batch length b (given, or floor(sqrt(n))), B = floor(n/b) batches covering the first B*b samples of
+ *     the window; a Welford pair (mb_c, M2b_c) of the B batch means.  Returned over the C chains:
+ *     batch_mean = sum_c mb_c / C, batch_within = sum_c M2b_c, batch_between = sum_c (mb_c - batch_mean)^2.
+ *   split halves: h = floor(n/2); half 1 = the first h samples of the window, half 2 = the last h (the middle sample
+ *     of an odd n belongs to neither).  Over the 2C half-chains, ordered (c, half 1), (c, half 2):
+ *     half_mean = mean of the half-chain means, half_within = sum M2, half_between = sum (m_hc - half_mean)^2.
+ * From these and var of sbd_posterior_stats:
+ *   tau2 = b (batch_within + B batch_between) / (C B - 1)   (NaN for C B < 2),
+ *   ESS = C n var / tau2,  MCSE = sqrt(tau2 / (C n)),
+ *   Rhat_split = sqrt(((h-1)/h W + Bh) / W),  W = half_within / (2C(h-1)),  Bh = half_between / (2C-1)
+ *                (NaN for h < 2).  DESIGN.md "Posterior statistics".
+ * ---------------------------------------------------------------------- */
+/* 0 (default): off.  -1: batch length floor(sqrt(n)).  b >= 1: batch length b.  Sticky, like sbd_set_posterior.
+   A run with diagnostics needs sbd_set_posterior(ctx, L >= 1); b > n gives B = 0 (zero batch arrays). */
+int sbd_set_posterior_diagnostics(sbd_ctx* ctx, int batch_len);
+/* diagnostics of the last run at block size 2^level; arrays ceil(rows/s) x ceil(cols/s), each nullable;
+   batch_len = b, n_batches = B, half_n = h of that run. */
+int sbd_posterior_diagnostics(const sbd_ctx* ctx, int level,
+                              double* batch_mean, double* batch_within, double* batch_between,
+                              double* half_mean, double* half_within, double* half_between,
+                              int* batch_len, int* n_batches, int* half_n);
+
+/* ------------------------------------------------------------------------
  * Launch-geometry control (no reference counterpart: the reference has no
  * launch geometry).  Used by the parity tests to pin the production geometry
  * of the fused Chambolle kernel at sizes the oracle finishes quickly, and by

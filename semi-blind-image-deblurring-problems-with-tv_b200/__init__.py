@@ -9,7 +9,7 @@ built library and a B200.
 """
 from ._lib import lib, LIB_PATH, SbdError, load_library  # noqa: F401
 from .host import (  # noqa: F401
-    Engine, engine_for, posterior_moments,
+    Engine, engine_for, posterior_moments, posterior_diagnostics,
     Gaussian_psf, psf_gaussian, psf_moffat, psf_laplace,
     moffat_psf, laplace_psf, gaussian_fft, diff_fftgaus_w1, diff_fftgaus_w2,
     diff_moffat_alpha, diff_moffat_beta, diff_laplace_b,

@@ -14,18 +14,91 @@
 
 namespace sbd {
 
+// ---- batch-means and split-half accumulators (DESIGN.md "Posterior statistics") ---------------------------------
+// Per chain and element (a pixel, or a block mean at s >= 2), for the sample v with window index k = ii - burnIn
+// (1 .. n), next to the window's Welford pair (m, M2):
+//   batch means  k <= B*b: bsum += v; at k = q*b: Y = bsum / b, Welford (mb, M2b) of Y with count q, bsum = 0.
+//                The n - B*b samples after the last batch are not batched.
+//   split halves half 1 is (m, M2) at k = h, copied there; half 2 is a Welford pair of k = n-h+1 .. n with count
+//                k - (n-h).  For odd n the middle sample belongs to neither.
+// Layout: bsum, mb, m2b like (m, M2), [chains][elements]; hm, hm2 [2*chains][elements] with half-chain 2c+half-1, so
+// that k_post_finalize over 2C "chains" forms the half-chain statistics in the order (c, half 1), (c, half 2).
+struct DiagAcc {
+    double *bsum, *mb, *m2b, *hm, *hm2;
+    int b, nbatch, h, n;                    // batch length b, batches B, half length h, window length n (per run)
+};
+
+// NE consecutive elements: one scalar, or two in one 16-byte access
+template <int NE>
+__device__ __forceinline__ void ld_n(const double* p, double (&v)[NE]) {
+    if constexpr (NE == 2) { const double2 t = *reinterpret_cast<const double2*>(p); v[0] = t.x; v[1] = t.y; }
+    else v[0] = *p;
+}
+template <int NE>
+__device__ __forceinline__ void st_n(double* p, const double (&v)[NE]) {
+    if constexpr (NE == 2) *reinterpret_cast<double2*>(p) = make_double2(v[0], v[1]);
+    else *p = v[0];
+}
+
+// Sample v of NE consecutive elements at idx in the chain arrays and hidx in half-chain 2c (2c+1 is `stride` further);
+// (mn, m2) is the window's Welford pair after v.  Every branch depends only on k and the run constants.
+template <int NE>
+__device__ __forceinline__ void diag_step(const DiagAcc& a, size_t idx, size_t hidx, size_t stride, int k,
+                                          const double (&v)[NE], const double (&mn)[NE], const double (&m2)[NE]) {
+    if (k <= a.nbatch * a.b) {
+        double s[NE];
+        ld_n(a.bsum + idx, s);
+#pragma unroll
+        for (int e = 0; e < NE; ++e) s[e] += v[e];
+        if (k % a.b == 0) {
+            const double inv = 1.0 / (double)(k / a.b);
+            double m[NE], q[NE];
+            ld_n(a.mb + idx, m); ld_n(a.m2b + idx, q);
+#pragma unroll
+            for (int e = 0; e < NE; ++e) {
+                const double y = s[e] / (double)a.b, d = y - m[e];
+                m[e] += d * inv;
+                q[e] += d * (y - m[e]);
+                s[e] = 0.0;
+            }
+            st_n(a.mb + idx, m); st_n(a.m2b + idx, q);
+        }
+        st_n(a.bsum + idx, s);
+    }
+    if (k == a.h) { st_n(a.hm + hidx, mn); st_n(a.hm2 + hidx, m2); }
+    const int k2 = k - (a.n - a.h);
+    if (k2 >= 1) {
+        const double inv = 1.0 / (double)k2;
+        double m[NE], q[NE];
+        ld_n(a.hm + hidx + stride, m); ld_n(a.hm2 + hidx + stride, q);
+#pragma unroll
+        for (int e = 0; e < NE; ++e) {
+            const double d = v[e] - m[e];
+            m[e] += d * inv;
+            q[e] += d * (v[e] - m[e]);
+        }
+        st_n(a.hm + hidx + stride, m); st_n(a.hm2 + hidx + stride, q);
+    }
+}
+
+// what k_langevin accumulates over the window ii = burnIn+1 .. samples besides the running mean
+enum { LGV_MEAN = 0, LGV_M2 = 1, LGV_DIAG = 2 };
+
 // X <- | X + gam*(P - X)/lamb - gam*Gf + sqrt(2 gam) Z |   (two elements per thread)
 // grid = (ceil(ceil(npix/2)/blockDim), n_chains)
 // An odd npix puts the element pairs of every other chain off the 16-byte grid: scalar accesses there, and the last
 // element of an image (a pair of its own) takes z0 of its pair (oracle/philox.py).
-// M2: also accumulate the per-chain sum of squared deviations (Welford) next to the running mean; post_m2 is then
+// LGV_M2: also accumulate the per-chain sum of squared deviations (Welford) next to the running mean; post_m2 is then
 // non-null whenever post_mean is.  The mean update is the same expression either way, so X_mean does not change.
-template <bool M2>
+// LGV_DIAG: M2 and the batch-means / split-half accumulators of `dg` (diag_step); unused by the other modes.
+template <int MODE>
 __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
                            const double* __restrict__ Gf, const double* __restrict__ noise,
-                           double* __restrict__ post_mean, double* __restrict__ post_m2, const Control* __restrict__ ctl,
+                           double* __restrict__ post_mean, double* __restrict__ post_m2, const DiagAcc dg,
+                           const Control* __restrict__ ctl,
                            double gam, double lamb, double sq2gam, size_t npix, int n_chains,
                            uint64_t seed, int chain_offset, int burnIn) {
+    constexpr bool M2 = MODE != LGV_MEAN, DIAG = MODE == LGV_DIAG;
     const size_t pair = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (2 * pair >= npix) return;
     const int ch = blockIdx.y;
@@ -50,7 +123,15 @@ __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
                 const double inv = 1.0 / (double)(ctl->ii - burnIn);
                 const double m = post_mean[off + e], d = r - m, mn = m + d * inv;
                 post_mean[off + e] = mn;
-                if (M2) post_m2[off + e] += d * (r - mn);
+                if (M2) {
+                    const double q = post_m2[off + e] + d * (r - mn);
+                    post_m2[off + e] = q;
+                    if (DIAG) {
+                        const double vr[1] = {r}, vm[1] = {mn}, vq[1] = {q};
+                        diag_step<1>(dg, off + e, 2 * (size_t)ch * npix + 2 * pair + e, npix, ctl->ii - burnIn,
+                                     vr, vm, vq);
+                    }
+                }
             }
         }
         return;
@@ -83,6 +164,10 @@ __global__ void k_langevin(double* __restrict__ X, const double* __restrict__ P,
             q.x += d.x * (r.x - m.x);
             q.y += d.y * (r.y - m.y);
             *reinterpret_cast<double2*>(post_m2 + off) = q;
+            if (DIAG) {
+                const double vr[2] = {r.x, r.y}, vm[2] = {m.x, m.y}, vq[2] = {q.x, q.y};
+                diag_step<2>(dg, off, 2 * (size_t)ch * npix + 2 * pair, npix, ctl->ii - burnIn, vr, vm, vq);
+            }
         }
     }
 }
@@ -255,7 +340,7 @@ __global__ void k_chain_mean(const double* __restrict__ in, double* __restrict__
 // ---- posterior moments at block sizes s = 2^j (DESIGN.md "Posterior statistics") --------------------------------
 // Per chain and block, Welford accumulators over the main-loop samples ii = burnIn+1 .. samples of the block mean
 // v = (sum of the block) / (pixels it contains):  d = v - m;  m += d / n_ii;  M2 += d (v - m),  n_ii = ii - burnIn.
-// j = 0 is the pixel scale (k_langevin<true>); k_post_blocks does j = 1 .. levels-1.
+// j = 0 is the pixel scale (k_langevin<LGV_M2>); k_post_blocks does j = 1 .. levels-1.
 constexpr int POST_MAXL = 7;                // block sizes 1 .. 64
 constexpr int POST_TILE = 64;               // pixels per side of the tile one thread block reduces
 struct PostGeom {
@@ -264,29 +349,43 @@ struct PostGeom {
     size_t off[POST_MAXL];                  // level j >= 1: offset of its [n_chains][bx*by] accumulators
 };
 
-__device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __restrict__ bm2, const PostGeom& g,
-                                             int j, int ch, int tx, int ty, int a, int b, double sum, double inv) {
+// DIAG: also the batch-means / split-half accumulators of dg (diag_step); their half-chain arrays of level j start at
+// 2 * off[j]
+template <bool DIAG>
+__device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __restrict__ bm2, const DiagAcc& dg,
+                                             const PostGeom& g, int j, int ch, int tx, int ty, int a, int b,
+                                             double sum, double inv, int k) {
     const int n = POST_TILE >> j, I = tx * n + a, J = ty * n + b;
     if (I >= g.bx[j] || J >= g.by[j]) return;
     const int s = 1 << j;
     const int cnt = (min((I + 1) * s, g.rows) - I * s) * (min((J + 1) * s, g.cols) - J * s);  // partial edge blocks
     const double v = sum / (double)cnt;
-    const size_t idx = g.off[j] + (size_t)ch * g.bx[j] * g.by[j] + (size_t)J * g.bx[j] + I;
+    const size_t nb = (size_t)g.bx[j] * g.by[j], e = (size_t)J * g.bx[j] + I;
+    const size_t idx = g.off[j] + (size_t)ch * nb + e;
     const double m = bm[idx], d = v - m, mn = m + d * inv;
     bm[idx] = mn;
-    bm2[idx] += d * (v - mn);
+    if (DIAG) {
+        const double q = bm2[idx] + d * (v - mn);
+        bm2[idx] = q;
+        const double vv[1] = {v}, vm[1] = {mn}, vq[1] = {q};
+        diag_step<1>(dg, idx, 2 * g.off[j] + 2 * (size_t)ch * nb + e, nb, k, vv, vm, vq);
+    } else {
+        bm2[idx] += d * (v - mn);
+    }
 }
 
 // One 64 x 64 tile of one chain's new sample per block, grid = (tiles, n_chains).  Level 1 sums 2 x 2 pixels read
 // straight from X, every further level sums 2 x 2 sums of the level below in shared memory, always as
 // (top-left + bottom-left) + (top-right + bottom-right) with zeros outside the image: the order depends only on
 // rows, cols and the level.  Runs only in the main loop after burn-in (Control, so a captured graph stays valid).
+template <bool DIAG>
 __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ X, double* __restrict__ bm,
-                                                     double* __restrict__ bm2, const PostGeom g,
+                                                     double* __restrict__ bm2, const DiagAcc dg, const PostGeom g,
                                                      const Control* __restrict__ ctl, int burnIn) {
     __shared__ double sm[32 * 32 + 16 * 16 + 8 * 8 + 4 * 4 + 2 * 2 + 1];
     if (!(ctl->phase == 1 && ctl->ii > burnIn)) return;
-    const double inv = 1.0 / (double)(ctl->ii - burnIn);
+    const int k = ctl->ii - burnIn;
+    const double inv = 1.0 / (double)k;
     const int ch = blockIdx.y, tx = blockIdx.x % g.tiles_x, ty = blockIdx.x / g.tiles_x;
     const int rows = g.rows, cols = g.cols;
     const double* x = X + (size_t)ch * rows * cols;
@@ -299,7 +398,7 @@ __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ 
         const double v01 = (i0 && j1) ? p[rows] : 0.0, v11 = (i1 && j1) ? p[rows + 1] : 0.0;
         const double sum = (v00 + v10) + (v01 + v11);
         sm[e] = sum;
-        post_welford(bm, bm2, g, 1, ch, tx, ty, a, b, sum, inv);
+        post_welford<DIAG>(bm, bm2, dg, g, 1, ch, tx, ty, a, b, sum, inv, k);
     }
     const double* prev = sm;
     double* cur = sm + 32 * 32;
@@ -313,7 +412,7 @@ __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ 
             const double* q = prev + 2 * b * n2 + 2 * a;
             const double sum = (q[0] + q[1]) + (q[n2] + q[n2 + 1]);
             cur[e] = sum;
-            post_welford(bm, bm2, g, lv, ch, tx, ty, a, b, sum, inv);
+            post_welford<DIAG>(bm, bm2, dg, g, lv, ch, tx, ty, a, b, sum, inv, k);
         }
         prev = cur;
         cur += n * n;

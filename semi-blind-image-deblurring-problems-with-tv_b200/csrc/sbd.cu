@@ -129,6 +129,12 @@ struct sbd_ctx {
     double* post_blk = nullptr; size_t post_blk_cap = 0;    // m and M2 of the levels >= 1, [2][sum_j n_chains*nb_j]
     double* post_out = nullptr; size_t post_out_cap = 0;    // mean, within, between of every level of the last run
     int stat_levels = 0, stat_n = 0, stat_chains = 0;       // what post_out holds (stat_levels 0: nothing)
+    // batch means and split halves (sbd_set_posterior_diagnostics / sbd_posterior_diagnostics, DiagAcc in sapg.cuh)
+    int post_diag = 0;                      // sticky request: 0 off, -1 batch length floor(sqrt(n)), b >= 1
+    double* diag_pix = nullptr; int diag_pix_batch = 0;     // pixel scale: 7 images per chain (DiagAcc layout)
+    double* diag_blk = nullptr; size_t diag_blk_cap = 0;    // levels >= 1: [7][sum_j n_chains*nb_j]
+    double* diag_out = nullptr; size_t diag_out_cap = 0;    // per level: batch mean/within/between, half mean/within/between
+    int diag_levels = 0, diag_b = 0, diag_nbatch = 0, diag_h = 0;   // what diag_out holds (diag_levels 0: nothing)
 
     // per-run scratch kept across calls (a cudaMalloc / cudaFree per sbd_sapg_run costs up to 0.6 s: a free tears down
     // whatever the driver deferred, e.g. the graphs of the run)
@@ -796,6 +802,43 @@ int sbd_posterior_stats(const sbd_ctx* ctx, int level, double* mean, double* wit
     SBD_CATCH(c)
 }
 
+int sbd_set_posterior_diagnostics(sbd_ctx* c, int batch_len) {
+    if (!c) return SBD_E_INVALID;
+    if (batch_len < -1) {
+        c->err = "sbd_set_posterior_diagnostics: batch_len must be 0 (off), -1 (floor(sqrt(n))) or a length >= 1";
+        return SBD_E_INVALID;
+    }
+    c->post_diag = batch_len;
+    return SBD_OK;
+}
+
+int sbd_posterior_diagnostics(const sbd_ctx* ctx, int level, double* batch_mean, double* batch_within,
+                              double* batch_between, double* half_mean, double* half_within, double* half_between,
+                              int* batch_len, int* n_batches, int* half_n) {
+    if (!ctx) return SBD_E_INVALID;
+    sbd_ctx* c = const_cast<sbd_ctx*>(ctx);     // only the error text and the stream are touched
+    SBD_TRY(c)
+    SBD_REQUIRE(c->diag_levels > 0, SBD_E_INVALID,
+                "sbd_posterior_diagnostics: the last SAPG run on this context accumulated no diagnostics "
+                "(sbd_set_posterior_diagnostics)");
+    SBD_REQUIRE(level >= 0 && level < c->diag_levels, SBD_E_INVALID,
+                "sbd_posterior_diagnostics: level " + std::to_string(level) + " outside 0.." +
+                std::to_string(c->diag_levels - 1) + " of the last run");
+    SBD_CUDA(cudaSetDevice(c->device));
+    size_t off = 0;
+    for (int j = 0; j < level; ++j) off += 6 * post_blocks(c, j);
+    const size_t nb = post_blocks(c, level);
+    double* dst[6] = {batch_mean, batch_within, batch_between, half_mean, half_within, half_between};
+    for (int q = 0; q < 6; ++q)
+        if (dst[q]) SBD_CUDA(cudaMemcpyAsync(dst[q], c->diag_out + off + q * nb, nb * sizeof(double),
+                                             cudaMemcpyDeviceToHost, c->stream));
+    SBD_CUDA(cudaStreamSynchronize(c->stream));
+    if (batch_len) *batch_len = c->diag_b;
+    if (n_batches) *n_batches = c->diag_nbatch;
+    if (half_n) *half_n = c->diag_h;
+    SBD_CATCH(c)
+}
+
 int sbd_set_option(sbd_ctx* c, const char* name, int value) {
     if (!c || !name) return SBD_E_INVALID;
     const std::string n(name);
@@ -952,6 +995,7 @@ int sbd_destroy(sbd_ctx* c) {
     dfree(c->tw_nx); dfree(c->tw_ny); dfree(c->taps); dfree(c->coef); dfree(c->ctl); dfree(c->psi_dev);
     dfree(c->ximg); dfree(c->yhat); dfree(c->allstats); dfree(c->post);
     dfree(c->post_m2); dfree(c->post_blk); dfree(c->post_out);
+    dfree(c->diag_pix); dfree(c->diag_blk); dfree(c->diag_out);
     dfree(c->trace_d); dfree(c->trace_i); dfree(c->sal_aty); dfree(c->sal_u); dfree(c->sal_bu); dfree(c->sal_xt);
     if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
     if (c->ev_langevin) cudaEventDestroy(c->ev_langevin);
@@ -1434,8 +1478,12 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     SBD_REQUIRE(prm->samples >= 1 && prm->warmup >= 0, SBD_E_INVALID, "sbd_sapg_run: samples >= 1, warmup >= 0");
     SBD_REQUIRE(prm->chambolle_maxiter >= 1, SBD_E_INVALID, "sbd_sapg_run: chambolle_maxiter >= 1");
     c->stat_levels = 0;
+    c->diag_levels = 0;
     SBD_REQUIRE(c->post_levels == 0 || prm->burnIn >= 1, SBD_E_INVALID,
                 "sbd_sapg_run: posterior statistics (sbd_set_posterior) need burnIn >= 1");
+    SBD_REQUIRE(c->post_diag == 0 || c->post_levels > 0, SBD_E_INVALID,
+                "sbd_sapg_run: posterior diagnostics (sbd_set_posterior_diagnostics) need the posterior statistics on "
+                "(sbd_set_posterior with levels >= 1)");
     const int ntot = std::max(prm->total_chains, nch);
     if (c->comm) SBD_REQUIRE(ntot == nch * c->nranks, SBD_E_INVALID, "sbd_sapg_run: total_chains must be n_chains * nranks");
     else SBD_REQUIRE(ntot == nch, SBD_E_COMM, "sbd_sapg_run: total_chains > n_chains needs sbd_comm_init");
@@ -1518,6 +1566,42 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
         if (out_elems > c->post_out_cap) { dfree(c->post_out); c->post_out = dalloc<double>(out_elems); c->post_out_cap = out_elems; }
         if (blk_half) SBD_CUDA(cudaMemsetAsync(c->post_blk, 0, sizeof(double) * 2 * blk_half, s));
     }
+    // batch means and split halves (DiagAcc): the pixel scale in diag_pix, the levels >= 1 in diag_blk, both laid out
+    // bsum, mb, m2b [nch][elements], hm, hm2 [2*nch][elements]
+    const bool diag = c->post_diag != 0;
+    DiagAcc dpix, dblk;
+    memset(&dpix, 0, sizeof dpix);
+    memset(&dblk, 0, sizeof dblk);
+    if (diag) {
+        const int n = std::max(samples - burnIn, 0);
+        int b = c->post_diag;
+        if (b < 0) {                            // floor(sqrt(n))
+            b = (int)std::sqrt((double)n);
+            while ((long long)b * b > n) --b;
+            while ((long long)(b + 1) * (b + 1) <= n) ++b;
+        }
+        dpix.b = b; dpix.nbatch = b > 0 ? n / b : 0; dpix.h = n / 2; dpix.n = n;
+        dblk.b = dpix.b; dblk.nbatch = dpix.nbatch; dblk.h = dpix.h; dblk.n = n;
+        const size_t img = (size_t)nch * c->npix;
+        if (c->diag_pix_batch < nch) {
+            dfree(c->diag_pix); c->diag_pix_batch = 0;          // stays consistent if the allocation throws
+            c->diag_pix = dalloc<double>(7 * img); c->diag_pix_batch = nch;
+        }
+        dpix.bsum = c->diag_pix; dpix.mb = dpix.bsum + img; dpix.m2b = dpix.mb + img;
+        dpix.hm = dpix.m2b + img; dpix.hm2 = dpix.hm + 2 * img;
+        SBD_CUDA(cudaMemsetAsync(c->diag_pix, 0, sizeof(double) * 7 * img, s));
+        if (7 * blk_half > c->diag_blk_cap) {
+            dfree(c->diag_blk); c->diag_blk_cap = 0;
+            c->diag_blk = dalloc<double>(7 * blk_half); c->diag_blk_cap = 7 * blk_half;
+        }
+        dblk.bsum = c->diag_blk; dblk.mb = dblk.bsum + blk_half; dblk.m2b = dblk.mb + blk_half;
+        dblk.hm = dblk.m2b + blk_half; dblk.hm2 = dblk.hm + 2 * blk_half;
+        if (blk_half) SBD_CUDA(cudaMemsetAsync(c->diag_blk, 0, sizeof(double) * 7 * blk_half, s));
+        if (2 * out_elems > c->diag_out_cap) {
+            dfree(c->diag_out); c->diag_out_cap = 0;
+            c->diag_out = dalloc<double>(2 * out_elems); c->diag_out_cap = 2 * out_elems;
+        }
+    }
 
     cudaEvent_t ev0, ev1;
     SBD_CUDA(cudaEventCreate(&ev0)); SBD_CUDA(cudaEventCreate(&ev1));
@@ -1576,14 +1660,18 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     auto unit = [&](int mode, bool grad_after) {
         { PhaseTimer pt(c, 1);
           const unsigned gx = (unsigned)(((c->npix + 1) / 2 + 255) / 256);
-          if (L > 0)
-              k_langevin<true><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->post_m2, c->ctl, k.gam,
-                                                             k.lamb, k.sq2gam, c->npix, nch, prm->seed, prm->chain_offset,
-                                                             burnIn);
+          if (diag)
+              k_langevin<LGV_DIAG><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->post_m2, dpix, c->ctl,
+                                                                 k.gam, k.lamb, k.sq2gam, c->npix, nch, prm->seed,
+                                                                 prm->chain_offset, burnIn);
+          else if (L > 0)
+              k_langevin<LGV_M2><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, c->post_m2, dpix, c->ctl,
+                                                               k.gam, k.lamb, k.sq2gam, c->npix, nch, prm->seed,
+                                                               prm->chain_offset, burnIn);
           else
-              k_langevin<false><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, nullptr, c->ctl, k.gam,
-                                                              k.lamb, k.sq2gam, c->npix, nch, prm->seed, prm->chain_offset,
-                                                              burnIn);
+              k_langevin<LGV_MEAN><<<dim3(gx, nch), 256, 0, s>>>(c->X, c->P, c->Gf, d_noise, post, nullptr, dpix, c->ctl,
+                                                                 k.gam, k.lamb, k.sq2gam, c->npix, nch, prm->seed,
+                                                                 prm->chain_offset, burnIn);
           LAUNCH_CHECK(c);
           if (mark_langevin) SBD_CUDA(cudaEventRecord(c->ev_langevin, s)); }
         const bool ov = c->opt_overlap != 0 && !c->profile;
@@ -1602,7 +1690,12 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
         }
         if (L >= 2 && mode == 2) {      // block moments of the new sample; reads X, like the prox next to it
             PhaseTimer pt(c, 1);
-            k_post_blocks<<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, pg, c->ctl, burnIn);
+            if (diag)
+                k_post_blocks<true><<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, dblk,
+                                                                          pg, c->ctl, burnIn);
+            else
+                k_post_blocks<false><<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, dblk,
+                                                                           pg, c->ctl, burnIn);
             LAUNCH_CHECK(c);
         }
         analyse(c, nch);
@@ -1741,6 +1834,21 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
             off += 3 * nb;
         }
     }
+    if (diag) {  // batch means over the nch chains, halves over the 2*nch half-chains (sbd_posterior_diagnostics)
+        size_t off = 0;
+        for (int j = 0; j < L; ++j) {
+            const size_t nb = post_blocks(c, j);
+            const DiagAcc& a = j == 0 ? dpix : dblk;
+            const size_t o = j == 0 ? 0 : pg.off[j];
+            double* r = c->diag_out + off;
+            k_post_finalize<<<(unsigned)((nb + 255) / 256), 256, 0, s>>>(a.mb + o, a.m2b + o, nb, nch, r, r + nb, r + 2 * nb);
+            LAUNCH_CHECK(c);
+            k_post_finalize<<<(unsigned)((nb + 255) / 256), 256, 0, s>>>(a.hm + 2 * o, a.hm2 + 2 * o, nb, 2 * nch, r + 3 * nb,
+                                                                        r + 4 * nb, r + 5 * nb);
+            LAUNCH_CHECK(c);
+            off += 6 * nb;
+        }
+    }
     SBD_CUDA(cudaStreamSynchronize(s));
     if (overlap_xlast) SBD_CUDA(cudaStreamSynchronize(c->copy_stream));
     if (dbg_host) fprintf(stderr, "[sbd] impl: read-back %.1f ms\n", now_ms() - H1);
@@ -1754,6 +1862,7 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     resolve_phase_events(c);
     out->last_samp = samples;                                       // Guassian.m:252 (no early break, Q10)
     if (L > 0) { c->stat_levels = L; c->stat_n = std::max(samples - burnIn, 0); c->stat_chains = nch; }
+    if (diag) { c->diag_levels = L; c->diag_b = dpix.b; c->diag_nbatch = dpix.nbatch; c->diag_h = dpix.h; }
 
     // ---- host post-processing of the scalar trajectories (Guassian.m:218-247,258-284)
     if (out->thetas) memcpy(out->thetas, th.data(), sizeof(double) * samples);

@@ -53,6 +53,34 @@ def posterior_moments(mean, within, between, n, chains):
     return var, np.sqrt(var), rhat
 
 
+def posterior_diagnostics(var, batch_within, batch_between, half_within, half_between, n, chains, batch_len,
+                          n_batches, half_n):
+    """ESS, MCSE and split-Rhat from the sufficient statistics sbd_posterior_diagnostics returns and var of
+    posterior_moments (DESIGN.md "Posterior statistics"): n samples per chain, `chains` chains, batch length b,
+    B = n_batches batches, half length h = half_n.
+      tau2 = b (batch_within + B batch_between) / (C B - 1)                (NaN for C B < 2)
+      ESS  = C n var / tau2,  MCSE = sqrt(tau2 / (C n))
+      W    = half_within / (2C(h-1)),  Bh = half_between / (2C-1),  Rhat_split = sqrt(((h-1)/h W + Bh) / W)
+                                                                          (NaN for h < 2)"""
+    var = np.asarray(var, dtype=np.float64)
+    n, C_, b, B, h = int(n), int(chains), int(batch_len), int(n_batches), int(half_n)
+    nan = np.full(var.shape, np.nan)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        if C_ * B >= 2:
+            tau2 = b * (np.asarray(batch_within, dtype=np.float64) + B * np.asarray(batch_between, dtype=np.float64)) \
+                / (C_ * B - 1)
+            ess, mcse = C_ * n * var / tau2, np.sqrt(tau2 / (C_ * n))
+        else:
+            ess, mcse = nan.copy(), nan.copy()
+        if h >= 2:
+            W = np.asarray(half_within, dtype=np.float64) / (2 * C_ * (h - 1))
+            Bh = np.asarray(half_between, dtype=np.float64) / (2 * C_ - 1)
+            rhat = np.sqrt(((h - 1) / h * W + Bh) / W)
+        else:
+            rhat = nan.copy()
+    return ess, mcse, rhat
+
+
 class Engine:
     """One libsbd context: fixed image size, PSF family and GPU."""
 
@@ -241,10 +269,36 @@ class Engine:
         return dict(scale=s, n=n.value, chains=ch.value, mean=mean, within=within, between=between, var=var, std=std,
                     Rhat=rhat)
 
-    def sapg(self, y, prm, X0=None, x_true=None, noise=None, want_X_warm=True, want_X_mean=False, post_levels=0):
+    def set_posterior_diagnostics(self, batch_len):
+        """sbd_set_posterior_diagnostics: 0 off, -1 batch length floor(sqrt(n)), b >= 1 batch length b; every
+        following run with posterior statistics also accumulates batch means and split halves (sticky)."""
+        self._check(lib.sbd_set_posterior_diagnostics(self._h, int(batch_len)))
+
+    def posterior_diagnostics(self, level, stats=None):
+        """Diagnostics of the last run at block size 2^level: dict(batch_mean, batch_within, batch_between, half_mean,
+        half_within, half_between, batch_len, n_batches, half_n, ESS, MCSE, Rhat_split), images ceil(rows/s) x
+        ceil(cols/s).  ESS and MCSE use var of `stats` (posterior_stats(level) of the same run, read if not given)."""
+        s = 1 << int(level)
+        bx, by = -(-self.rows // s), -(-self.cols // s)
+        bufs = [np.zeros(bx * by) for _ in range(6)]
+        b, nb, h = C.c_int(), C.c_int(), C.c_int()
+        self._check(lib.sbd_posterior_diagnostics(self._h, int(level), *[_p(q) for q in bufs], C.byref(b),
+                                                  C.byref(nb), C.byref(h)))
+        names = ("batch_mean", "batch_within", "batch_between", "half_mean", "half_within", "half_between")
+        d = {k: q.reshape(by, bx).T.copy() for k, q in zip(names, bufs)}
+        d.update(batch_len=b.value, n_batches=nb.value, half_n=h.value)
+        st = self.posterior_stats(level) if stats is None else stats
+        d["ESS"], d["MCSE"], d["Rhat_split"] = posterior_diagnostics(
+            st["var"], d["batch_within"], d["batch_between"], d["half_within"], d["half_between"], st["n"],
+            st["chains"], b.value, nb.value, h.value)
+        return d
+
+    def sapg(self, y, prm, X0=None, x_true=None, noise=None, want_X_warm=True, want_X_mean=False, post_levels=0,
+             post_batch=0):
         """Run sbd_sapg_run.  `prm` is a filled sbd_params; noise (optional)
         is [(warmup-1)+(samples-1), n_chains, rows, cols].  post_levels L > 0 adds out["posterior"]: one
-        `posterior_stats` dict per block size 1 .. 2^(L-1); the context is left with the statistics off."""
+        `posterior_stats` dict per block size 1 .. 2^(L-1); post_batch (-1: floor(sqrt(n)), b >= 1; needs L > 0)
+        adds the `posterior_diagnostics` fields to each.  The context is left with both off."""
         yb, _ = self._img(y, "y")
         x0b = self._img(X0, "X0")[0] if X0 is not None else None
         xtb = self._img(x_true, "x_true")[0] if x_true is not None else None
@@ -278,11 +332,17 @@ class Engine:
             xm = np.zeros(self.rows * self.cols); tr.X_mean = _p(xm)
         self.set_posterior(post_levels)
         try:
+            self.set_posterior_diagnostics(post_batch)
             self._check(lib.sbd_sapg_run(self._h, _p(yb), _p(x0b), _p(xtb), C.byref(prm), _p(nb), C.byref(tr)))
             posterior = [self.posterior_stats(j) for j in range(int(post_levels))]
+            if post_batch:
+                for j, st in enumerate(posterior):
+                    st.update(self.posterior_diagnostics(j, st))
         finally:
             if post_levels:
                 lib.sbd_set_posterior(self._h, 0)
+            if post_batch:
+                lib.sbd_set_posterior_diagnostics(self._h, 0)
         out = dict(bufs)
         if post_levels:
             out["posterior"] = posterior
@@ -513,7 +573,10 @@ def make_params(model, op, c=None, n_chains=1, seed=1, chain_offset=0, total_cha
     return p
 
 
-def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, x_true=None, post_levels=0):
+def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, x_true=None, post_levels=0,
+         post_batch=0):
+    if int(post_batch) < -1:
+        raise ValueError(f"post_batch must be 0 (off), -1 (floor(sqrt(n))) or a batch length >= 1, got {post_batch}")
     y = np.asarray(y, dtype=np.float64)
     op = dict(op)
     if "warmup" not in op:
@@ -521,7 +584,8 @@ def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean
     prm = make_params(model, op, c, n_chains=n_chains, seed=seed, post_mean=post_mean)
     eng = engine or engine_for(y.shape, op["psf_size"], model, op.get("phi", 0.0), max_batch=n_chains)
     X0 = op.get("X0")                                                           # Guassian.m:10-12
-    out = eng.sapg(y, prm, X0=X0, x_true=x_true, noise=noise, want_X_mean=post_mean, post_levels=post_levels)
+    out = eng.sapg(y, prm, X0=X0, x_true=x_true, noise=noise, want_X_mean=post_mean, post_levels=post_levels,
+                   post_batch=post_batch)
     return op, prm, out
 
 
@@ -531,16 +595,21 @@ def _add_posterior(r, o):
     if "posterior" in o:
         p0 = o["posterior"][0]
         r.update(posterior=o["posterior"], posteriorvar=p0["var"], posteriorstd=p0["std"], Rhat=p0["Rhat"])
+        if "ESS" in p0:                         # post_batch
+            r.update(ESS=p0["ESS"], MCSE=p0["MCSE"], Rhat_split=p0["Rhat_split"])
     return r
 
 
-def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
+def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
+                            post_batch=0):
     """[theta_EB, w1_EB, w2_EB, sigma_EB, results] = SAPG_algorithm_Guassian(y, op, c)
     SAPG/SAPG_algorithm_Guassian.m:7-308.  `op` must carry the plain-data fields
     the reference already stores (psf_size, phi, lambda, gamma, ...); the function
     handles in `op` are not used - the engine implements the model they encode.  post_levels > 0 adds the posterior
-    statistics (Engine.sapg) as results["posterior"], ["posteriorvar"], ["posteriorstd"], ["Rhat"]."""
-    op, prm, o = _run(GAUSSIAN, y, op, c, noise, n_chains, seed, engine, post_mean, post_levels=post_levels)
+    statistics (Engine.sapg) as results["posterior"], ["posteriorvar"], ["posteriorstd"], ["Rhat"]; post_batch
+    (-1 or b >= 1, with post_levels) adds the pixel-scale results["ESS"], ["MCSE"], ["Rhat_split"]."""
+    op, prm, o = _run(GAUSSIAN, y, op, c, noise, n_chains, seed, engine, post_mean, post_levels=post_levels,
+                      post_batch=post_batch)
     r = dict(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindParameters=o["seconds"], last_samp=o["last_samp"],
              logPiTraceX=o["logPiTraceX"], gXTrace=o["gXTrace"],
              theta_EB=o["EB"][0], last_theta=o["thetas"][-1], thetas=o["thetas"], mean_thetas=o["mean_theta"],
@@ -557,10 +626,12 @@ def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=Non
     return r["theta_EB"], r["w1_EB"], r["w2_EB"], r["sigma_EB"], r
 
 
-def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
+def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
+                          post_batch=0):
     """[theta_EB, alpha_EB, beta_EB, sigma2_EB, results] = SAPG_algorithm_moffat(y, op)
     SAPG/SAPG_algorithm_moffat.m:7-297."""
-    op, prm, o = _run(MOFFAT, y, op, None, noise, n_chains, seed, engine, post_mean, post_levels=post_levels)
+    op, prm, o = _run(MOFFAT, y, op, None, noise, n_chains, seed, engine, post_mean, post_levels=post_levels,
+                      post_batch=post_batch)
     err_psf = o["err_psf"].copy(); err_psf[0] = 0.0          # err_psf(1) is never assigned (moffat.m:205)
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],
@@ -580,13 +651,14 @@ def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, po
     return r["mean_theta"], r["alpha_EB"], r["beta_EB"], r["sigma_EB"], r
 
 
-def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0):
+def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
+                           post_batch=0):
     """[theta_EB, b_EB, sigma_EB, results] = SAPG_algorithm_laplace(y, op)
     SAPG/SAPG_algorithm_laplace.m:7-268 (needs op.x, the ground truth, :28)."""
     if "x" not in op:
         raise KeyError("Reference to non-existent field 'x'.")                 # laplace.m:28
     op, prm, o = _run(LAPLACE, y, op, None, noise, n_chains, seed, engine, post_mean, x_true=op["x"],
-                      post_levels=post_levels)
+                      post_levels=post_levels, post_batch=post_batch)
     err_warm = np.zeros(max(int(op["warmup"]), 1)); err_warm[0] = o["err_warm0"]    # laplace.m:28-29
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],

@@ -51,5 +51,6 @@ if isfield(op, 'seed'), P.seed = op.seed; end
 P.use_graph = -1;                                                    % automatic: CUDA-graph replay for small images
 if isfield(op, 'use_graph'), P.use_graph = op.use_graph; end
 if isfield(op, 'post_levels'), P.post_levels = op.post_levels; end   % posterior statistics (sbd_posterior.m)
+if isfield(op, 'post_batch'), P.post_batch = op.post_batch; end      % their ESS / MCSE / split Rhat (-1: auto)
 r2res = names;
 end

@@ -21,7 +21,10 @@
  *   r       = sbd_mex('sapg', y, X0, xtrue, model, t, phi, P, noise)      SAPG/SAPG_algorithm_*.m
  *             P.post_levels = L (optional, 0 = off) adds r.posterior: a 1x1 struct with one field per block size,
  *             s1, s2, s4, ..., each a struct with scale, n, chains, mean, within, between, var, std, Rhat
- *             (include/sbd.h sbd_posterior_stats; the .m wrappers turn it into a struct array)
+ *             (include/sbd.h sbd_posterior_stats; the .m wrappers turn it into a struct array).
+ *             P.post_batch = b (optional, 0 = off; -1: floor(sqrt(n)), b >= 1: batch length b; needs post_levels)
+ *             adds batch_mean, batch_within, batch_between, half_mean, half_within, half_between, batch_len,
+ *             n_batches, half_n, ESS, MCSE, Rhat_split to each (sbd_posterior_diagnostics)
  *   [v,k]   = sbd_mex('max_eigenval', [M N], model, t, phi, psi, tol, maxit, x0)   utils/max_eigenval_*.m
  *   [y,s,n] = sbd_mex('observe', x, model, t, phi, psi, bsnr, noise)      run_Gaussian_demo.m:145-168
  *   [x,obj,dist,mses] = sbd_mex('salsa', y, model, t, phi, psi, tau, mu, maxiter, tolA, tviters, xtrue)
@@ -105,9 +108,11 @@ static mxArray* vec(int n, double** p) {
 }
 
 /* posterior statistics of the last run at block sizes 1 .. 2^(levels-1), with var, std and Rhat formed as DESIGN.md
-   states them ("Posterior statistics") */
-static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels) {
-    static const char* fields[] = {"scale", "n", "chains", "mean", "within", "between", "var", "std", "Rhat"};
+   states them ("Posterior statistics"); diag: also the diagnostics with ESS, MCSE and Rhat_split */
+static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels, int diag) {
+    static const char* fields[] = {"scale", "n", "chains", "mean", "within", "between", "var", "std", "Rhat",
+                                   "batch_mean", "batch_within", "batch_between", "half_mean", "half_within",
+                                   "half_between", "batch_len", "n_batches", "half_n", "ESS", "MCSE", "Rhat_split"};
     char lnames[8][8];
     const char* lp[8];
     mxArray* out;
@@ -116,7 +121,7 @@ static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels) {
     out = mxCreateStructMatrix(1, 1, levels, lp);
     for (j = 0; j < levels; ++j) {
         const int s = 1 << j, bx = (rows + s - 1) / s, by = (cols + s - 1) / s;
-        mxArray* e = mxCreateStructMatrix(1, 1, 9, fields);
+        mxArray* e = mxCreateStructMatrix(1, 1, diag ? 21 : 9, fields);
         mxArray *a[6];
         double* p[6];
         int q, n = 0, C = 0;
@@ -136,6 +141,26 @@ static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels) {
         mxSetField(e, 0, "chains", mxCreateDoubleScalar((double)C));
         mxSetField(e, 0, "mean", a[0]); mxSetField(e, 0, "within", a[1]); mxSetField(e, 0, "between", a[2]);
         mxSetField(e, 0, "var", a[3]); mxSetField(e, 0, "std", a[4]); mxSetField(e, 0, "Rhat", a[5]);
+        if (diag) {
+            mxArray* d[9];
+            double* g[9];
+            int b = 0, B = 0, h = 0;
+            for (q = 0; q < 9; ++q) { d[q] = mxCreateDoubleMatrix(bx, by, mxREAL); g[q] = mxGetPr(d[q]); }
+            rc = sbd_posterior_diagnostics(c, j, g[0], g[1], g[2], g[3], g[4], g[5], &b, &B, &h);
+            if (rc) { sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); fail(c, "sbd_posterior_diagnostics", rc); }
+            for (i = 0; i < (size_t)bx * by; ++i) {
+                const double tau2 = C * B >= 2 ? b * (g[1][i] + B * g[2][i]) / (C * (double)B - 1.0) : NAN;
+                const double Wh = g[4][i] / (2.0 * C * (h - 1.0)), Bh = g[5][i] / (2.0 * C - 1.0);
+                g[6][i] = C * (double)n * p[3][i] / tau2;                                /* ESS */
+                g[7][i] = sqrt(tau2 / (C * (double)n));                                  /* MCSE */
+                g[8][i] = h >= 2 ? sqrt(((h - 1.0) / h * Wh + Bh) / Wh) : NAN;           /* split Rhat */
+            }
+            for (q = 0; q < 6; ++q) mxSetField(e, 0, fields[9 + q], d[q]);
+            mxSetField(e, 0, "batch_len", mxCreateDoubleScalar((double)b));
+            mxSetField(e, 0, "n_batches", mxCreateDoubleScalar((double)B));
+            mxSetField(e, 0, "half_n", mxCreateDoubleScalar((double)h));
+            mxSetField(e, 0, "ESS", d[6]); mxSetField(e, 0, "MCSE", d[7]); mxSetField(e, 0, "Rhat_split", d[8]);
+        }
         mxSetField(out, 0, lp[j], e);
     }
     return out;
@@ -233,7 +258,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         sbd_traces t;
         sbd_ctx* c;
         double* q[21];
-        int i, nm, levels;
+        int i, nm, levels, batch;
         mxArray* r;
         if (!mxIsStruct(P)) mexErrMsgIdAndTxt("sbd:type", "P must be a struct");
         memset(&p, 0, sizeof p); memset(&t, 0, sizeof t);
@@ -255,6 +280,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         p.seed = (uint64_t)field(P, "seed", 0, 1); p.chain_offset = 0; p.total_chains = p.n_chains;
         p.use_graph = (int)field(P, "use_graph", 0, -1);            /* -1: automatic (CUDA graph for small problems) */
         levels = (int)field(P, "post_levels", 0, 0);                 /* posterior statistics, 0 = off */
+        batch = (int)field(P, "post_batch", 0, 0);                   /* their diagnostics, 0 = off */
         c = get_ctx(rows, cols, (int)mxGetScalar(prhs[5]), (int)mxGetScalar(prhs[4]), mxGetScalar(prhs[6]), p.n_chains);
         nm = p.samples - p.burnIn; if (nm < 0) nm = 0;
         /* the `posterior` field exists only when it was asked for: otherwise the old field set */
@@ -271,12 +297,14 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         { mxArray* a = mxCreateDoubleMatrix(rows, cols * p.n_chains, mxREAL); t.X_warm = mxGetPr(a); mxSetField(r, 0, "X_warm", a); }
         { mxArray* a = mxCreateDoubleMatrix(rows, cols * p.n_chains, mxREAL); t.X_last = mxGetPr(a); mxSetField(r, 0, "X_last", a); }
         if ((rc = sbd_set_posterior(c, levels))) fail(c, "sbd_set_posterior", rc);
+        if ((rc = sbd_set_posterior_diagnostics(c, batch))) { sbd_set_posterior(c, 0); fail(c, "sbd_set_posterior_diagnostics", rc); }
         rc = sbd_sapg_run(c, y, X0, xt, &p, noise, &t);
-        if (rc) { sbd_set_posterior(c, 0); fail(c, "sbd_sapg_run", rc); }
+        if (rc) { sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); fail(c, "sbd_sapg_run", rc); }
         if (levels > 0) {
             mxArray* post;
-            post = posterior_struct(c, rows, cols, levels);
-            sbd_set_posterior(c, 0);                             /* cached context: the request is sticky */
+            post = posterior_struct(c, rows, cols, levels, batch != 0);
+            sbd_set_posterior(c, 0);                             /* cached context: the requests are sticky */
+            sbd_set_posterior_diagnostics(c, 0);
             mxSetField(r, 0, "posterior", post);
         }
         { double* e; mxSetField(r, 0, "EB", vec(4, &e)); for (i = 0; i < 4; ++i) e[i] = t.EB[i]; }

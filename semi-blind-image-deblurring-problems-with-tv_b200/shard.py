@@ -83,40 +83,70 @@ class ChainShard:
             mean = sum_r C_r mean_r / C,  within = sum_r within_r,  between = sum_r [between_r + C_r (mean_r - mean)^2]
         This is exact algebra, but it sums in another order than one context running all C chains, so the result
         equals a one-GPU run to rounding (~1e-13 relative), not bit for bit.  Returns the same list of dicts with
-        var, std and Rhat recomputed from the merged statistics."""
-        from .host import posterior_moments
+        var, std and Rhat recomputed from the merged statistics.
+        With the diagnostics (Engine.sapg(..., post_batch=b)) the batch statistics are merged the same way with
+        weights C_r and the half statistics with weights 2 C_r, and ESS, MCSE and Rhat_split are recomputed; the
+        ranks must agree in n, batch_len and n_batches."""
+        from .host import posterior_moments, posterior_diagnostics
         out = []
         for st in stats:
-            mean = np.asarray(st["mean"], dtype=np.float64)
-            local = np.stack([mean, np.asarray(st["within"], dtype=np.float64),
-                              np.asarray(st["between"], dtype=np.float64)])
+            diag = "batch_mean" in st
+            keys = ("mean", "within", "between") + (DIAG_KEYS if diag else ())
+            local = np.stack([np.asarray(st[k], dtype=np.float64) for k in keys])
+            meta = [int(st["chains"]), int(st["n"]), int(diag)]
+            if diag:
+                meta += [int(st["batch_len"]), int(st["n_batches"]), int(st["half_n"])]
             if self.world_size == 1:
-                parts, counts, ns = [local], [int(st["chains"])], [int(st["n"])]
+                parts, metas = [local], [meta]
             else:
                 import torch
                 import torch.distributed as dist
+                mt = torch.tensor(meta + [0] * (6 - len(meta)), dtype=torch.int64)
+                mts = [torch.empty_like(mt) for _ in range(self.world_size)]
+                dist.all_gather(mts, mt)
+                metas = [[int(v) for v in m] for m in mts]
+                if len({m[2] for m in metas}) != 1:
+                    raise ValueError("combine_posterior: some ranks have diagnostics and some do not")
                 mine = torch.from_numpy(np.ascontiguousarray(local))
                 gathered = [torch.empty_like(mine) for _ in range(self.world_size)]
                 dist.all_gather(gathered, mine)
-                meta = torch.tensor([int(st["chains"]), int(st["n"])], dtype=torch.int64)
-                metas = [torch.empty_like(meta) for _ in range(self.world_size)]
-                dist.all_gather(metas, meta)
                 parts = [g.numpy() for g in gathered]
-                counts = [int(m[0]) for m in metas]
-                ns = [int(m[1]) for m in metas]
+            counts = [m[0] for m in metas]
+            ns = [m[1] for m in metas]
             if len(set(ns)) != 1:
                 raise ValueError(f"combine_posterior: ranks differ in samples per chain {ns}")
             C_ = sum(counts)
-            tot = np.zeros_like(mean)
-            for cr, pr in zip(counts, parts):              # rank order
-                tot = tot + cr * pr[0]
-            m = tot / C_
-            within = np.zeros_like(mean)
-            between = np.zeros_like(mean)
-            for cr, pr in zip(counts, parts):
-                within = within + pr[1]
-                between = between + (pr[2] + cr * (pr[0] - m) ** 2)
+            m, within, between = _merge(counts, [p[0:3] for p in parts])
             var, std, rhat = posterior_moments(m, within, between, ns[0], C_)
-            out.append(dict(scale=st["scale"], n=ns[0], chains=C_, mean=m, within=within, between=between, var=var,
-                            std=std, Rhat=rhat))
+            d = dict(scale=st["scale"], n=ns[0], chains=C_, mean=m, within=within, between=between, var=var,
+                     std=std, Rhat=rhat)
+            if diag:
+                bs = {tuple(mm[3:6]) for mm in metas}
+                if len(bs) != 1:
+                    raise ValueError(f"combine_posterior: ranks differ in (batch_len, n_batches, half_n) {sorted(bs)}")
+                b, B, h = bs.pop()
+                merged = _merge(counts, [p[3:6] for p in parts]) + _merge([2 * c for c in counts], [p[6:9] for p in parts])
+                d.update(zip(DIAG_KEYS, merged))
+                d.update(batch_len=b, n_batches=B, half_n=h)
+                d["ESS"], d["MCSE"], d["Rhat_split"] = posterior_diagnostics(
+                    var, d["batch_within"], d["batch_between"], d["half_within"], d["half_between"], ns[0], C_, b, B, h)
+            out.append(d)
         return out
+
+
+DIAG_KEYS = ("batch_mean", "batch_within", "batch_between", "half_mean", "half_within", "half_between")
+
+
+def _merge(counts, parts):
+    """(mean, within, between) of groups of counts[r] members each, from their own (mean_r, within_r, between_r),
+    summed in rank order"""
+    tot = np.zeros_like(parts[0][0])
+    for cr, pr in zip(counts, parts):
+        tot = tot + cr * pr[0]
+    m = tot / sum(counts)
+    within = np.zeros_like(m)
+    between = np.zeros_like(m)
+    for cr, pr in zip(counts, parts):
+        within = within + pr[1]
+        between = between + (pr[2] + cr * (pr[0] - m) ** 2)
+    return m, within, between

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Cost of the posterior statistics (sbd_set_posterior) in the SAPG main loop.
+"""Cost of the posterior statistics (sbd_set_posterior) and their diagnostics (sbd_set_posterior_diagnostics) in the
+SAPG main loop.
 
-For each configuration the same seeded problem is run with the statistics off, with post_mean only, and with
-post_levels L = 1 and L = 4, alternating the variants; each variant reports the best of --reps runs of the
+For each configuration the same seeded problem is run with the statistics off, with post_mean only, with
+post_levels L = 1 and L = 4, and with L = 4 plus the diagnostics at the automatic batch length, alternating the variants; each variant reports the best of --reps runs of the
 device-timed main loop (sbd_traces.seconds_main) as chain-steps/s.  The runs go through sbd_sapg_run_dev with y in
 HBM and no trace or sample copies, so only the main loop is timed.  The card's name, power limit and max SM clock
 are printed with the numbers.
@@ -23,7 +24,8 @@ sys.path.insert(0, ROOT)
 
 # (rows, cols, chains, use_graph, main-loop steps)
 CONFIGS = [(4096, 4096, 8, 0, 12), (2160, 3840, 8, 0, 12), (512, 512, 1, 0, 200), (256, 256, 1, 1, 400)]
-VARIANTS = [("off", 0, 0), ("post_mean", 1, 0), ("L1", 0, 1), ("L4", 0, 4)]     # (name, post_mean, post_levels)
+# (name, post_mean, post_levels, post_batch)
+VARIANTS = [("off", 0, 0, 0), ("post_mean", 1, 0, 0), ("L1", 0, 1, 0), ("L4", 0, 4, 0), ("L4_diag", 0, 4, -1)]
 
 
 def gpu_info():
@@ -66,11 +68,13 @@ def main():
         y = (128 + 40 * torch.randn(cols, rows, generator=g, dtype=torch.float64)).abs().cuda()   # column-major image
         best = {v[0]: 0.0 for v in VARIANTS}
         for rep in range(a.reps + 1):                    # rep 0 warms every variant up (allocations, graphs)
-            for name, pm, L in VARIANTS:
+            for name, pm, L, b in VARIANTS:
                 prm = params(H, rows, cols, nch, steps, use_graph, pm)
                 tr = sbd_traces()
                 eng._check(lib.sbd_set_posterior(eng._h, L))
+                eng._check(lib.sbd_set_posterior_diagnostics(eng._h, b))
                 eng._check(lib.sbd_sapg_run_dev(eng._h, C.c_void_p(y.data_ptr()), None, C.byref(prm), C.byref(tr)))
+                eng._check(lib.sbd_set_posterior_diagnostics(eng._h, 0))
                 eng._check(lib.sbd_set_posterior(eng._h, 0))
                 rate = steps * nch / tr.seconds_main
                 if rep > 0:
@@ -79,6 +83,7 @@ def main():
                    **{f"chain_steps_per_s_{k}": v for k, v in best.items()})
         row["overhead_L1_vs_post_mean"] = best["post_mean"] / best["L1"] - 1
         row["overhead_L4_vs_post_mean"] = best["post_mean"] / best["L4"] - 1
+        row["overhead_L4_diag_vs_L4"] = best["L4"] / best["L4_diag"] - 1
         print(json.dumps(row), flush=True)
         rows_out.append(row)
         eng.close()
