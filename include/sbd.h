@@ -316,6 +316,23 @@ int sbd_posterior_diagnostics(const sbd_ctx* ctx, int level,
                               int* batch_len, int* n_batches, int* half_n);
 
 /* ------------------------------------------------------------------------
+ * Marginal credible intervals and the posterior median (no reference counterpart).  Over the same window and block
+ * sizes, one streaming estimator per element fed the values of the C chains of this context at every step, in local
+ * chain order (N = C*n values): extended P^2 (Jain & Chlamtac 1985, Raatikainen 1987) with 9 markers at the
+ * probabilities {0, a/4, a/2, 1/4+a/4, 1/2, 3/4-a/4, 1-a/2, 1-a/4, 1}, a = alpha.  lower = quantile alpha/2,
+ * median = 1/2, upper = 1 - alpha/2: the markers q2, q4, q6 for N >= 9; for 1 <= N < 9 the linear interpolation of the
+ * N sorted values at h = (N-1)p; NaN for N = 0.  Memory does not grow with C.  DESIGN.md "Credible intervals and the
+ * median".
+ * ---------------------------------------------------------------------- */
+/* 0 (default): off.  0 < alpha < 1: every following SAPG run accumulates the posterior quantiles alpha/2, 1/2,
+   1 - alpha/2 at the block sizes of sbd_set_posterior.  Sticky.  Needs sbd_set_posterior(ctx, L >= 1). */
+int sbd_set_posterior_quantiles(sbd_ctx* ctx, double alpha);
+/* lower, median, upper of the last run at block size 2^level (each nullable, ceil(rows/s) x ceil(cols/s));
+   alpha and count = C*n of that run. */
+int sbd_posterior_quantiles(const sbd_ctx* ctx, int level, double* lower, double* median, double* upper,
+                            double* alpha, long long* count);
+
+/* ------------------------------------------------------------------------
  * Launch-geometry control (no reference counterpart: the reference has no
  * launch geometry).  Used by the parity tests to pin the production geometry
  * of the fused Chambolle kernel at sizes the oracle finishes quickly, and by

@@ -100,6 +100,8 @@ SIGNATURES = {
     "sbd_posterior_stats": (C.c_int, [C.c_void_p, C.c_int, c_double_p, c_double_p, c_double_p, c_int_p, c_int_p]),
     "sbd_set_posterior_diagnostics": (C.c_int, [C.c_void_p, C.c_int]),
     "sbd_posterior_diagnostics": (C.c_int, [C.c_void_p, C.c_int] + [c_double_p] * 6 + [c_int_p] * 3),
+    "sbd_set_posterior_quantiles": (C.c_int, [C.c_void_p, C.c_double]),
+    "sbd_posterior_quantiles": (C.c_int, [C.c_void_p, C.c_int] + [c_double_p] * 4 + [C.POINTER(C.c_longlong)]),
     "sbd_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),
     "sbd_get_geometry": (C.c_int, [C.c_void_p, C.c_int, c_int_p]),
 }

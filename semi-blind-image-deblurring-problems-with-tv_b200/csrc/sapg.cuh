@@ -350,11 +350,11 @@ struct PostGeom {
 };
 
 // DIAG: also the batch-means / split-half accumulators of dg (diag_step); their half-chain arrays of level j start at
-// 2 * off[j]
-template <bool DIAG>
+// 2 * off[j].  QUANT: also store the block mean v into qv (layout of bm) for k_post_quantile.
+template <bool DIAG, bool QUANT>
 __device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __restrict__ bm2, const DiagAcc& dg,
-                                             const PostGeom& g, int j, int ch, int tx, int ty, int a, int b,
-                                             double sum, double inv, int k) {
+                                             double* __restrict__ qv, const PostGeom& g, int j, int ch, int tx, int ty,
+                                             int a, int b, double sum, double inv, int k) {
     const int n = POST_TILE >> j, I = tx * n + a, J = ty * n + b;
     if (I >= g.bx[j] || J >= g.by[j]) return;
     const int s = 1 << j;
@@ -362,6 +362,7 @@ __device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __
     const double v = sum / (double)cnt;
     const size_t nb = (size_t)g.bx[j] * g.by[j], e = (size_t)J * g.bx[j] + I;
     const size_t idx = g.off[j] + (size_t)ch * nb + e;
+    if (QUANT) qv[idx] = v;
     const double m = bm[idx], d = v - m, mn = m + d * inv;
     bm[idx] = mn;
     if (DIAG) {
@@ -378,9 +379,10 @@ __device__ __forceinline__ void post_welford(double* __restrict__ bm, double* __
 // straight from X, every further level sums 2 x 2 sums of the level below in shared memory, always as
 // (top-left + bottom-left) + (top-right + bottom-right) with zeros outside the image: the order depends only on
 // rows, cols and the level.  Runs only in the main loop after burn-in (Control, so a captured graph stays valid).
-template <bool DIAG>
+template <bool DIAG, bool QUANT>
 __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ X, double* __restrict__ bm,
-                                                     double* __restrict__ bm2, const DiagAcc dg, const PostGeom g,
+                                                     double* __restrict__ bm2, const DiagAcc dg,
+                                                     double* __restrict__ qv, const PostGeom g,
                                                      const Control* __restrict__ ctl, int burnIn) {
     __shared__ double sm[32 * 32 + 16 * 16 + 8 * 8 + 4 * 4 + 2 * 2 + 1];
     if (!(ctl->phase == 1 && ctl->ii > burnIn)) return;
@@ -398,7 +400,7 @@ __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ 
         const double v01 = (i0 && j1) ? p[rows] : 0.0, v11 = (i1 && j1) ? p[rows + 1] : 0.0;
         const double sum = (v00 + v10) + (v01 + v11);
         sm[e] = sum;
-        post_welford<DIAG>(bm, bm2, dg, g, 1, ch, tx, ty, a, b, sum, inv, k);
+        post_welford<DIAG, QUANT>(bm, bm2, dg, qv, g, 1, ch, tx, ty, a, b, sum, inv, k);
     }
     const double* prev = sm;
     double* cur = sm + 32 * 32;
@@ -412,7 +414,7 @@ __global__ void __launch_bounds__(256) k_post_blocks(const double* __restrict__ 
             const double* q = prev + 2 * b * n2 + 2 * a;
             const double sum = (q[0] + q[1]) + (q[n2] + q[n2 + 1]);
             cur[e] = sum;
-            post_welford<DIAG>(bm, bm2, dg, g, lv, ch, tx, ty, a, b, sum, inv, k);
+            post_welford<DIAG, QUANT>(bm, bm2, dg, qv, g, lv, ch, tx, ty, a, b, sum, inv, k);
         }
         prev = cur;
         cur += n * n;
@@ -435,6 +437,123 @@ __global__ void k_post_finalize(const double* __restrict__ m, const double* __re
         b += d * d;
     }
     mean[i] = mu; within[i] = w; between[i] = b;
+}
+
+// ---- posterior quantiles: extended P^2 (DESIGN.md "Credible intervals and the median") --------------------------
+// One estimator per element of every level (not per chain): at each main-loop step after burn-in the values of the C
+// chains are fed in local chain order, so after k window steps it has seen N = C*k values.  9 markers, heights q_i and
+// integer positions n_i with desired positions 1 + (N-1) f_i.  N <= 9: q holds the values sorted.  Every expression is
+// that of tests/posterior_quantile_oracle.py, evaluated with __d*_rn (no FMA contraction), so both agree bitwise.
+// State SoA over the E elements of all levels: q [9][E], np [7][E] (n_1 .. n_7; n_0 = 1 and n_8 = N are implied).
+struct QuantAcc {
+    double* q;
+    int* np;
+    double f[9];                            // marker probabilities, formed on the host
+    size_t E;                               // elements of all levels
+    int levels;
+    size_t start[POST_MAXL];                // first element of level j
+    size_t nb[POST_MAXL];                   // elements of level j = chain stride of its values
+    const double* src[POST_MAXL];           // values of level j: X (j = 0), block means of k_post_blocks (j >= 1)
+};
+
+// one thread per element of all levels; grid = ceil(E / 256).  Runs only in the main loop after burn-in (Control).
+__global__ void __launch_bounds__(256) k_post_quantile(const QuantAcc a, const Control* __restrict__ ctl, int burnIn,
+                                                       int n_chains) {
+    if (!(ctl->phase == 1 && ctl->ii > burnIn)) return;
+    const size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= a.E) return;
+    const double* src = a.src[0];
+    size_t nb = a.nb[0], le = e;
+#pragma unroll      // constant level indices: the QuantAcc arrays stay in the parameter bank
+    for (int j = 1; j < POST_MAXL; ++j)
+        if (j < a.levels && e >= a.start[j]) { src = a.src[j]; nb = a.nb[j]; le = e - a.start[j]; }
+    int N = (ctl->ii - burnIn - 1) * n_chains;      // values seen before this step (C*n < 2^31: checked on the host)
+    double q[9];
+    int n[9];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) q[i] = a.q[(size_t)i * a.E + e];
+#pragma unroll
+    for (int i = 1; i < 8; ++i) n[i] = a.np[(size_t)(i - 1) * a.E + e];
+    n[0] = 1;
+    for (int c = 0; c < n_chains; ++c, ++N) {
+        const double x = __ldg(src + (size_t)c * nb + le);
+        if (N < 9) {                                // insertion: q[0..N] sorted, x after the values <= x
+#pragma unroll
+            for (int i = 8; i >= 0; --i) {
+                if (i <= N) {
+                    const bool keep = i < N && q[i] <= x;
+                    const bool shift = i >= 1 && q[i >= 1 ? i - 1 : 0] > x;
+                    q[i] = keep ? q[i] : (shift ? q[i >= 1 ? i - 1 : 0] : x);
+                }
+            }
+            if (N == 8) {
+#pragma unroll
+                for (int i = 1; i < 8; ++i) n[i] = i + 1;
+            }
+            continue;
+        }
+        int k = 0;
+        if (x < q[0]) { q[0] = x; k = 0; }
+        else if (x >= q[8]) { q[8] = x; k = 7; }
+        else {
+#pragma unroll
+            for (int i = 1; i < 8; ++i) if (q[i] <= x) k = i;
+        }
+#pragma unroll
+        for (int i = 1; i < 8; ++i) n[i] += i > k;
+        n[8] = N + 1;                               // the count after x
+        const double Nm1 = (double)N;               // (N+1) - 1
+#pragma unroll
+        for (int i = 1; i < 8; ++i) {
+            const double d = __dsub_rn(__dadd_rn(1.0, __dmul_rn(Nm1, a.f[i])), (double)n[i]);
+            const int dr = n[i + 1] - n[i], dl = n[i] - n[i - 1];
+            if ((d >= 1.0 && dr > 1) || (d <= -1.0 && dl > 1)) {
+                // parabolic prediction over one common denominator: one division per moving marker instead of three
+                // (the markers of a warp move in different iterations; profiles/r06_posterior_quantiles.md)
+                const int s = d >= 1.0 ? 1 : -1;
+                const double sd = (double)s, ndr = (double)dr, ndl = (double)dl;
+                const double dq1 = __dsub_rn(q[i + 1], q[i]), dq0 = __dsub_rn(q[i], q[i - 1]);
+                const double num = __dadd_rn(__dmul_rn(__dmul_rn(__dadd_rn(ndl, sd), ndl), dq1),
+                                             __dmul_rn(__dmul_rn(__dsub_rn(ndr, sd), ndr), dq0));
+                const double den = __dmul_rn(__dmul_rn(ndr, ndl), __dadd_rn(ndr, ndl));
+                const double qp = __dadd_rn(q[i], __ddiv_rn(__dmul_rn(sd, num), den));
+                if (q[i - 1] < qp && qp < q[i + 1]) q[i] = qp;
+                else q[i] = __dadd_rn(q[i], __dmul_rn(sd, s > 0 ? __ddiv_rn(dq1, ndr) : __ddiv_rn(dq0, ndl)));
+                n[i] += s;
+            }
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < 9; ++i) a.q[(size_t)i * a.E + e] = q[i];
+#pragma unroll
+    for (int i = 1; i < 8; ++i) a.np[(size_t)(i - 1) * a.E + e] = n[i];
+}
+
+// lower / median / upper (probabilities p[0..2]) of the nb elements of one level starting at element e0 after N
+// values: N >= 9 the markers q_2, q_4, q_6; 1 <= N < 9 the linear interpolation of the sorted values
+// v[h] + (h - floor h)(v[h+1] - v[h]), h = (N-1) p; N = 0 NaN
+__global__ void k_post_quantile_finalize(const double* __restrict__ q, size_t E, size_t e0, size_t nb, int N,
+                                         double p0, double p1, double p2, double* __restrict__ lower,
+                                         double* __restrict__ median, double* __restrict__ upper) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nb) return;
+    const double* v = q + e0 + i;
+    const double p[3] = {p0, p1, p2};
+    double r[3];
+#pragma unroll
+    for (int t = 0; t < 3; ++t) {
+        if (N >= 9) {
+            r[t] = v[(size_t)(2 + 2 * t) * E];
+        } else if (N == 0) {
+            r[t] = __longlong_as_double(0x7ff8000000000000LL);
+        } else {
+            const double h = __dmul_rn((double)(N - 1), p[t]), fl = floor(h), fr = __dsub_rn(h, fl);
+            const int lo = (int)fl;
+            const double vl = v[(size_t)lo * E];
+            r[t] = fr == 0.0 ? vl : __dadd_rn(vl, __dmul_rn(fr, __dsub_rn(v[(size_t)(lo + 1) * E], vl)));
+        }
+    }
+    lower[i] = r[0]; median[i] = r[1]; upper[i] = r[2];
 }
 
 // sum of x over one image -> out[0]   (mean(mean(Ax)), run_Gaussian_demo.m:148)

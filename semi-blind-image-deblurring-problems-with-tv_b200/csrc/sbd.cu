@@ -135,6 +135,12 @@ struct sbd_ctx {
     double* diag_blk = nullptr; size_t diag_blk_cap = 0;    // levels >= 1: [7][sum_j n_chains*nb_j]
     double* diag_out = nullptr; size_t diag_out_cap = 0;    // per level: batch mean/within/between, half mean/within/between
     int diag_levels = 0, diag_b = 0, diag_nbatch = 0, diag_h = 0;   // what diag_out holds (diag_levels 0: nothing)
+    // credible intervals and median (sbd_set_posterior_quantiles / sbd_posterior_quantiles, QuantAcc in sapg.cuh)
+    double post_ci = 0.0;                   // sticky request: 0 off, else the credible level alpha in (0, 1)
+    double* quant_q = nullptr; int* quant_n = nullptr; size_t quant_cap = 0;   // P^2 state [9][E], [7][E]
+    double* quant_blk = nullptr; size_t quant_blk_cap = 0;  // block means of the current sample, post_blk layout
+    double* quant_out = nullptr; size_t quant_out_cap = 0;  // lower, median, upper of every level of the last run
+    int quant_levels = 0; double quant_alpha = 0.0; long long quant_count = 0;   // what quant_out holds
 
     // per-run scratch kept across calls (a cudaMalloc / cudaFree per sbd_sapg_run costs up to 0.6 s: a free tears down
     // whatever the driver deferred, e.g. the graphs of the run)
@@ -839,6 +845,41 @@ int sbd_posterior_diagnostics(const sbd_ctx* ctx, int level, double* batch_mean,
     SBD_CATCH(c)
 }
 
+int sbd_set_posterior_quantiles(sbd_ctx* c, double alpha) {
+    if (!c) return SBD_E_INVALID;
+    if (!(alpha >= 0.0 && alpha < 1.0)) {
+        c->err = "sbd_set_posterior_quantiles: alpha must be 0 (off) or a credible level in (0, 1)";
+        return SBD_E_INVALID;
+    }
+    c->post_ci = alpha;
+    return SBD_OK;
+}
+
+int sbd_posterior_quantiles(const sbd_ctx* ctx, int level, double* lower, double* median, double* upper,
+                            double* alpha, long long* count) {
+    if (!ctx) return SBD_E_INVALID;
+    sbd_ctx* c = const_cast<sbd_ctx*>(ctx);     // only the error text and the stream are touched
+    SBD_TRY(c)
+    SBD_REQUIRE(c->quant_levels > 0, SBD_E_INVALID,
+                "sbd_posterior_quantiles: the last SAPG run on this context accumulated no quantiles "
+                "(sbd_set_posterior_quantiles)");
+    SBD_REQUIRE(level >= 0 && level < c->quant_levels, SBD_E_INVALID,
+                "sbd_posterior_quantiles: level " + std::to_string(level) + " outside 0.." +
+                std::to_string(c->quant_levels - 1) + " of the last run");
+    SBD_CUDA(cudaSetDevice(c->device));
+    size_t off = 0;
+    for (int j = 0; j < level; ++j) off += 3 * post_blocks(c, j);
+    const size_t nb = post_blocks(c, level);
+    double* dst[3] = {lower, median, upper};
+    for (int q = 0; q < 3; ++q)
+        if (dst[q]) SBD_CUDA(cudaMemcpyAsync(dst[q], c->quant_out + off + q * nb, nb * sizeof(double),
+                                             cudaMemcpyDeviceToHost, c->stream));
+    SBD_CUDA(cudaStreamSynchronize(c->stream));
+    if (alpha) *alpha = c->quant_alpha;
+    if (count) *count = c->quant_count;
+    SBD_CATCH(c)
+}
+
 int sbd_set_option(sbd_ctx* c, const char* name, int value) {
     if (!c || !name) return SBD_E_INVALID;
     const std::string n(name);
@@ -996,6 +1037,7 @@ int sbd_destroy(sbd_ctx* c) {
     dfree(c->ximg); dfree(c->yhat); dfree(c->allstats); dfree(c->post);
     dfree(c->post_m2); dfree(c->post_blk); dfree(c->post_out);
     dfree(c->diag_pix); dfree(c->diag_blk); dfree(c->diag_out);
+    dfree(c->quant_q); dfree(c->quant_n); dfree(c->quant_blk); dfree(c->quant_out);
     dfree(c->trace_d); dfree(c->trace_i); dfree(c->sal_aty); dfree(c->sal_u); dfree(c->sal_bu); dfree(c->sal_xt);
     if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
     if (c->ev_langevin) cudaEventDestroy(c->ev_langevin);
@@ -1479,11 +1521,18 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     SBD_REQUIRE(prm->chambolle_maxiter >= 1, SBD_E_INVALID, "sbd_sapg_run: chambolle_maxiter >= 1");
     c->stat_levels = 0;
     c->diag_levels = 0;
+    c->quant_levels = 0;
     SBD_REQUIRE(c->post_levels == 0 || prm->burnIn >= 1, SBD_E_INVALID,
                 "sbd_sapg_run: posterior statistics (sbd_set_posterior) need burnIn >= 1");
     SBD_REQUIRE(c->post_diag == 0 || c->post_levels > 0, SBD_E_INVALID,
                 "sbd_sapg_run: posterior diagnostics (sbd_set_posterior_diagnostics) need the posterior statistics on "
                 "(sbd_set_posterior with levels >= 1)");
+    SBD_REQUIRE(c->post_ci == 0.0 || c->post_levels > 0, SBD_E_INVALID,
+                "sbd_sapg_run: posterior quantiles (sbd_set_posterior_quantiles) need the posterior statistics on "
+                "(sbd_set_posterior with levels >= 1)");
+    SBD_REQUIRE(c->post_ci == 0.0 ||
+                (long long)nch * std::max(prm->samples - prm->burnIn, 0) < (1LL << 31), SBD_E_INVALID,
+                "sbd_sapg_run: posterior quantiles need n_chains * (samples - burnIn) < 2^31 (int32 marker positions)");
     const int ntot = std::max(prm->total_chains, nch);
     if (c->comm) SBD_REQUIRE(ntot == nch * c->nranks, SBD_E_INVALID, "sbd_sapg_run: total_chains must be n_chains * nranks");
     else SBD_REQUIRE(ntot == nch, SBD_E_COMM, "sbd_sapg_run: total_chains > n_chains needs sbd_comm_init");
@@ -1602,6 +1651,37 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
             c->diag_out = dalloc<double>(2 * out_elems); c->diag_out_cap = 2 * out_elems;
         }
     }
+    // credible intervals and median (QuantAcc): P^2 state over the E elements of all levels, the pixel scale read
+    // from X, the levels >= 1 from the block means k_post_blocks<., true> stores in quant_blk (post_blk layout)
+    const bool quant = c->post_ci != 0.0;
+    QuantAcc qa;
+    memset(&qa, 0, sizeof qa);
+    double qp[3] = {0.0, 0.0, 0.0};         // lower, median, upper = f[2], f[4], f[6]
+    if (quant) {
+        const double al = c->post_ci;
+        const double f[9] = {0.0, al / 4, al / 2, 0.25 + al / 4, 0.5, 0.75 - al / 4, 1 - al / 2, 1 - al / 4, 1.0};
+        for (int i = 0; i < 9; ++i) qa.f[i] = f[i];
+        qp[0] = f[2]; qp[1] = f[4]; qp[2] = f[6];
+        qa.levels = L;
+        for (int j = 0; j < L; ++j) {
+            qa.start[j] = qa.E; qa.nb[j] = post_blocks(c, j); qa.E += qa.nb[j];
+        }
+        if (qa.E > c->quant_cap) {
+            dfree(c->quant_q); dfree(c->quant_n); c->quant_cap = 0;     // stays consistent if an allocation throws
+            c->quant_q = dalloc<double>(9 * qa.E); c->quant_n = dalloc<int>(7 * qa.E); c->quant_cap = qa.E;
+        }
+        if (blk_half > c->quant_blk_cap) {
+            dfree(c->quant_blk); c->quant_blk_cap = 0;
+            c->quant_blk = dalloc<double>(blk_half); c->quant_blk_cap = blk_half;
+        }
+        if (out_elems > c->quant_out_cap) {
+            dfree(c->quant_out); c->quant_out_cap = 0;
+            c->quant_out = dalloc<double>(out_elems); c->quant_out_cap = out_elems;
+        }
+        qa.q = c->quant_q; qa.np = c->quant_n;
+        qa.src[0] = c->X;
+        for (int j = 1; j < L; ++j) qa.src[j] = c->quant_blk + pg.off[j];
+    }
 
     cudaEvent_t ev0, ev1;
     SBD_CUDA(cudaEventCreate(&ev0)); SBD_CUDA(cudaEventCreate(&ev1));
@@ -1690,12 +1770,15 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
         }
         if (L >= 2 && mode == 2) {      // block moments of the new sample; reads X, like the prox next to it
             PhaseTimer pt(c, 1);
-            if (diag)
-                k_post_blocks<true><<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, dblk,
-                                                                          pg, c->ctl, burnIn);
-            else
-                k_post_blocks<false><<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, dblk,
-                                                                           pg, c->ctl, burnIn);
+            auto kb = diag ? (quant ? k_post_blocks<true, true> : k_post_blocks<true, false>)
+                           : (quant ? k_post_blocks<false, true> : k_post_blocks<false, false>);
+            kb<<<dim3(post_tiles, nch), 256, 0, s>>>(c->X, c->post_blk, c->post_blk + blk_half, dblk, c->quant_blk, pg,
+                                                     c->ctl, burnIn);
+            LAUNCH_CHECK(c);
+        }
+        if (quant && mode == 2) {       // P^2 markers of every element; reads X and the block means just stored
+            PhaseTimer pt(c, 1);
+            k_post_quantile<<<(unsigned)((qa.E + 255) / 256), 256, 0, s>>>(qa, c->ctl, burnIn, nch);
             LAUNCH_CHECK(c);
         }
         analyse(c, nch);
@@ -1849,6 +1932,18 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
             off += 6 * nb;
         }
     }
+    const long long qcount = (long long)nch * std::max(samples - burnIn, 0);
+    if (quant) {  // lower / median / upper per level (sbd_posterior_quantiles)
+        size_t off = 0;
+        for (int j = 0; j < L; ++j) {
+            const size_t nb = qa.nb[j];
+            double* r = c->quant_out + off;
+            k_post_quantile_finalize<<<(unsigned)((nb + 255) / 256), 256, 0, s>>>(
+                qa.q, qa.E, qa.start[j], nb, (int)qcount, qp[0], qp[1], qp[2], r, r + nb, r + 2 * nb);
+            LAUNCH_CHECK(c);
+            off += 3 * nb;
+        }
+    }
     SBD_CUDA(cudaStreamSynchronize(s));
     if (overlap_xlast) SBD_CUDA(cudaStreamSynchronize(c->copy_stream));
     if (dbg_host) fprintf(stderr, "[sbd] impl: read-back %.1f ms\n", now_ms() - H1);
@@ -1863,6 +1958,7 @@ void sapg_run_impl(sbd_ctx* c, const double* d_y, const double* d_X0, const doub
     out->last_samp = samples;                                       // Guassian.m:252 (no early break, Q10)
     if (L > 0) { c->stat_levels = L; c->stat_n = std::max(samples - burnIn, 0); c->stat_chains = nch; }
     if (diag) { c->diag_levels = L; c->diag_b = dpix.b; c->diag_nbatch = dpix.nbatch; c->diag_h = dpix.h; }
+    if (quant) { c->quant_levels = L; c->quant_alpha = c->post_ci; c->quant_count = qcount; }
 
     // ---- host post-processing of the scalar trajectories (Guassian.m:218-247,258-284)
     if (out->thetas) memcpy(out->thetas, th.data(), sizeof(double) * samples);

@@ -83,11 +83,12 @@ def setup_demo(model, x, engine=None, noise=None, x0_eig=None, seed=1, chambolle
 
 
 def run_demo(model, x, engine=None, map_estimate=True, n_chains=1, seed=1, noise_sapg=None, post_mean=False,
-             use_graph=True, name="", post_levels=0, post_batch=0, **kw):
+             use_graph=True, name="", post_levels=0, post_batch=0, post_ci=0.0, **kw):
     """One pass of the body of the experiment loops (run_Gaussian_demo.m:100-242): observation, SAPG,
     SALSA MAP estimate with the empirical-Bayes parameters, MSE.  Returns the `results` dict the script
     saves, plus timings.  post_levels > 0 adds the posterior statistics (host.Engine.sapg), post_batch (-1 or a batch
-    length, with post_levels) their ESS, MCSE and split-Rhat."""
+    length, with post_levels) their ESS, MCSE and split-Rhat, post_ci = alpha (with post_levels) the median and the
+    (1 - alpha) credible interval."""
     t0 = time.perf_counter()
     y, op, eng = setup_demo(model, x, engine=engine, seed=seed, **kw)
     if n_chains > eng.max_batch:
@@ -98,17 +99,17 @@ def run_demo(model, x, engine=None, map_estimate=True, n_chains=1, seed=1, noise
     if model == H.GAUSSIAN:
         th, p0, p1, s2, r = H.SAPG_algorithm_Guassian(y, op, dict(C_GAUSSIAN), noise=noise_sapg, n_chains=n_chains,
                                                       seed=seed, engine=eng, post_mean=post_mean,
-                                                      post_levels=post_levels, post_batch=post_batch)
+                                                      post_levels=post_levels, post_batch=post_batch, post_ci=post_ci)
         psi_eb = (p0, p1)
     elif model == H.MOFFAT:
         th, p0, p1, s2, r = H.SAPG_algorithm_moffat(y, op, noise=noise_sapg, n_chains=n_chains, seed=seed, engine=eng,
                                                     post_mean=post_mean, post_levels=post_levels,
-                                                    post_batch=post_batch)
+                                                    post_batch=post_batch, post_ci=post_ci)
         psi_eb = (p0, p1)
     else:
         th, p0, s2, r = H.SAPG_algorithm_laplace(y, op, noise=noise_sapg, n_chains=n_chains, seed=seed, engine=eng,
                                                  post_mean=post_mean, post_levels=post_levels,
-                                                 post_batch=post_batch)
+                                                 post_batch=post_batch, post_ci=post_ci)
         psi_eb = (p0,)
     t2 = time.perf_counter()
     res = dict(r)
@@ -144,6 +145,8 @@ def _savable(res):
                 if "ESS" in p:                  # post_batch
                     for q in ("ESS", "MCSE", "Rhat_split"):
                         out[f"{q}_s{p['scale']}"] = p[q]
+                if "ci_width" in p:             # post_ci
+                    out[f"CI_width_s{p['scale']}"] = p["ci_width"]
     return out
 
 

@@ -293,12 +293,31 @@ class Engine:
             st["chains"], b.value, nb.value, h.value)
         return d
 
+    def set_posterior_quantiles(self, alpha):
+        """sbd_set_posterior_quantiles: 0 off, 0 < alpha < 1: every following run with posterior statistics also
+        accumulates the quantiles alpha/2, 1/2, 1 - alpha/2 (P^2 on the device; sticky)."""
+        self._check(lib.sbd_set_posterior_quantiles(self._h, float(alpha)))
+
+    def posterior_quantiles(self, level):
+        """Credible interval and median of the last run at block size 2^level: dict(ci_alpha, ci_count, lower, median,
+        upper, ci_width = upper - lower), images ceil(rows/s) x ceil(cols/s); ci_count = C*n values per element."""
+        s = 1 << int(level)
+        bx, by = -(-self.rows // s), -(-self.cols // s)
+        bufs = [np.zeros(bx * by) for _ in range(3)]
+        al, cnt = C.c_double(), C.c_longlong()
+        self._check(lib.sbd_posterior_quantiles(self._h, int(level), *[_p(q) for q in bufs], C.byref(al),
+                                                C.byref(cnt)))
+        lower, median, upper = (q.reshape(by, bx).T.copy() for q in bufs)
+        return dict(ci_alpha=al.value, ci_count=int(cnt.value), lower=lower, median=median, upper=upper,
+                    ci_width=upper - lower)
+
     def sapg(self, y, prm, X0=None, x_true=None, noise=None, want_X_warm=True, want_X_mean=False, post_levels=0,
-             post_batch=0):
+             post_batch=0, post_ci=0.0):
         """Run sbd_sapg_run.  `prm` is a filled sbd_params; noise (optional)
         is [(warmup-1)+(samples-1), n_chains, rows, cols].  post_levels L > 0 adds out["posterior"]: one
         `posterior_stats` dict per block size 1 .. 2^(L-1); post_batch (-1: floor(sqrt(n)), b >= 1; needs L > 0)
-        adds the `posterior_diagnostics` fields to each.  The context is left with both off."""
+        adds the `posterior_diagnostics` fields to each, post_ci = alpha (0 < alpha < 1; needs L > 0) the
+        `posterior_quantiles` fields.  The context is left with all three off."""
         yb, _ = self._img(y, "y")
         x0b = self._img(X0, "X0")[0] if X0 is not None else None
         xtb = self._img(x_true, "x_true")[0] if x_true is not None else None
@@ -333,16 +352,22 @@ class Engine:
         self.set_posterior(post_levels)
         try:
             self.set_posterior_diagnostics(post_batch)
+            self.set_posterior_quantiles(post_ci)
             self._check(lib.sbd_sapg_run(self._h, _p(yb), _p(x0b), _p(xtb), C.byref(prm), _p(nb), C.byref(tr)))
             posterior = [self.posterior_stats(j) for j in range(int(post_levels))]
             if post_batch:
                 for j, st in enumerate(posterior):
                     st.update(self.posterior_diagnostics(j, st))
+            if post_ci:
+                for j, st in enumerate(posterior):
+                    st.update(self.posterior_quantiles(j))
         finally:
             if post_levels:
                 lib.sbd_set_posterior(self._h, 0)
             if post_batch:
                 lib.sbd_set_posterior_diagnostics(self._h, 0)
+            if post_ci:
+                lib.sbd_set_posterior_quantiles(self._h, 0.0)
         out = dict(bufs)
         if post_levels:
             out["posterior"] = posterior
@@ -574,9 +599,11 @@ def make_params(model, op, c=None, n_chains=1, seed=1, chain_offset=0, total_cha
 
 
 def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, x_true=None, post_levels=0,
-         post_batch=0):
+         post_batch=0, post_ci=0.0):
     if int(post_batch) < -1:
         raise ValueError(f"post_batch must be 0 (off), -1 (floor(sqrt(n))) or a batch length >= 1, got {post_batch}")
+    if not 0.0 <= float(post_ci) < 1.0:
+        raise ValueError(f"post_ci must be 0 (off) or a credible level alpha in (0, 1), got {post_ci}")
     y = np.asarray(y, dtype=np.float64)
     op = dict(op)
     if "warmup" not in op:
@@ -585,7 +612,7 @@ def _run(model, y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean
     eng = engine or engine_for(y.shape, op["psf_size"], model, op.get("phi", 0.0), max_batch=n_chains)
     X0 = op.get("X0")                                                           # Guassian.m:10-12
     out = eng.sapg(y, prm, X0=X0, x_true=x_true, noise=noise, want_X_mean=post_mean, post_levels=post_levels,
-                   post_batch=post_batch)
+                   post_batch=post_batch, post_ci=post_ci)
     return op, prm, out
 
 
@@ -597,19 +624,23 @@ def _add_posterior(r, o):
         r.update(posterior=o["posterior"], posteriorvar=p0["var"], posteriorstd=p0["std"], Rhat=p0["Rhat"])
         if "ESS" in p0:                         # post_batch
             r.update(ESS=p0["ESS"], MCSE=p0["MCSE"], Rhat_split=p0["Rhat_split"])
+        if "median" in p0:                      # post_ci
+            r.update(posteriormedian=p0["median"], CI_lower=p0["lower"], CI_upper=p0["upper"])
     return r
 
 
 def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
-                            post_batch=0):
+                            post_batch=0, post_ci=0.0):
     """[theta_EB, w1_EB, w2_EB, sigma_EB, results] = SAPG_algorithm_Guassian(y, op, c)
     SAPG/SAPG_algorithm_Guassian.m:7-308.  `op` must carry the plain-data fields
     the reference already stores (psf_size, phi, lambda, gamma, ...); the function
     handles in `op` are not used - the engine implements the model they encode.  post_levels > 0 adds the posterior
     statistics (Engine.sapg) as results["posterior"], ["posteriorvar"], ["posteriorstd"], ["Rhat"]; post_batch
-    (-1 or b >= 1, with post_levels) adds the pixel-scale results["ESS"], ["MCSE"], ["Rhat_split"]."""
+    (-1 or b >= 1, with post_levels) adds the pixel-scale results["ESS"], ["MCSE"], ["Rhat_split"]; post_ci = alpha
+    (0 < alpha < 1, with post_levels) the pixel-scale results["posteriormedian"], ["CI_lower"], ["CI_upper"] of the
+    (1 - alpha) credible interval."""
     op, prm, o = _run(GAUSSIAN, y, op, c, noise, n_chains, seed, engine, post_mean, post_levels=post_levels,
-                      post_batch=post_batch)
+                      post_batch=post_batch, post_ci=post_ci)
     r = dict(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindParameters=o["seconds"], last_samp=o["last_samp"],
              logPiTraceX=o["logPiTraceX"], gXTrace=o["gXTrace"],
              theta_EB=o["EB"][0], last_theta=o["thetas"][-1], thetas=o["thetas"], mean_thetas=o["mean_theta"],
@@ -627,11 +658,11 @@ def SAPG_algorithm_Guassian(y, op, c, noise=None, n_chains=1, seed=1, engine=Non
 
 
 def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
-                          post_batch=0):
+                          post_batch=0, post_ci=0.0):
     """[theta_EB, alpha_EB, beta_EB, sigma2_EB, results] = SAPG_algorithm_moffat(y, op)
     SAPG/SAPG_algorithm_moffat.m:7-297."""
     op, prm, o = _run(MOFFAT, y, op, None, noise, n_chains, seed, engine, post_mean, post_levels=post_levels,
-                      post_batch=post_batch)
+                      post_batch=post_batch, post_ci=post_ci)
     err_psf = o["err_psf"].copy(); err_psf[0] = 0.0          # err_psf(1) is never assigned (moffat.m:205)
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],
@@ -652,13 +683,13 @@ def SAPG_algorithm_moffat(y, op, noise=None, n_chains=1, seed=1, engine=None, po
 
 
 def SAPG_algorithm_laplace(y, op, noise=None, n_chains=1, seed=1, engine=None, post_mean=False, post_levels=0,
-                           post_batch=0):
+                           post_batch=0, post_ci=0.0):
     """[theta_EB, b_EB, sigma_EB, results] = SAPG_algorithm_laplace(y, op)
     SAPG/SAPG_algorithm_laplace.m:7-268 (needs op.x, the ground truth, :28)."""
     if "x" not in op:
         raise KeyError("Reference to non-existent field 'x'.")                 # laplace.m:28
     op, prm, o = _run(LAPLACE, y, op, None, noise, n_chains, seed, engine, post_mean, x_true=op["x"],
-                      post_levels=post_levels, post_batch=post_batch)
+                      post_levels=post_levels, post_batch=post_batch, post_ci=post_ci)
     err_warm = np.zeros(max(int(op["warmup"]), 1)); err_warm[0] = o["err_warm0"]    # laplace.m:28-29
     r = {"lambda": op["lambda"], "gamma": op["gamma"]}
     r.update(logPiTrace_WU=o["logPiTrace_WU"], execTimeFindTheta=o["seconds"], last_samp=o["last_samp"],

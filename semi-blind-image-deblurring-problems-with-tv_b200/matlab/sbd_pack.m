@@ -52,5 +52,6 @@ P.use_graph = -1;                                                    % automatic
 if isfield(op, 'use_graph'), P.use_graph = op.use_graph; end
 if isfield(op, 'post_levels'), P.post_levels = op.post_levels; end   % posterior statistics (sbd_posterior.m)
 if isfield(op, 'post_batch'), P.post_batch = op.post_batch; end      % their ESS / MCSE / split Rhat (-1: auto)
+if isfield(op, 'post_ci'), P.post_ci = op.post_ci; end               % median and 1 - alpha credible interval
 r2res = names;
 end

@@ -8,6 +8,9 @@ function results = sbd_posterior(results, r)
 % and, with op.post_batch (sbd_posterior_diagnostics), the struct array also has the fields batch_mean, batch_within,
 % batch_between, half_mean, half_within, half_between, batch_len, n_batches, half_n, ESS, MCSE, Rhat_split, and
 %   results.ESS, results.MCSE, results.Rhat_split                 their pixel-scale (s = 1) values
+% and, with op.post_ci = alpha (sbd_posterior_quantiles), the fields ci_alpha, ci_count, lower, median, upper,
+% ci_width (the 1 - alpha credible interval and the posterior median), and
+%   results.posteriormedian, results.CI_lower, results.CI_upper   their pixel-scale (s = 1) values
 f = fieldnames(r.posterior);
 for k = 1:numel(f)
     post(k) = r.posterior.(f{k});
@@ -16,5 +19,8 @@ results.posterior = post;
 results.posteriorvar = post(1).var; results.posteriorstd = post(1).std; results.Rhat = post(1).Rhat;
 if isfield(post, 'ESS')
     results.ESS = post(1).ESS; results.MCSE = post(1).MCSE; results.Rhat_split = post(1).Rhat_split;
+end
+if isfield(post, 'median')
+    results.posteriormedian = post(1).median; results.CI_lower = post(1).lower; results.CI_upper = post(1).upper;
 end
 end

@@ -25,6 +25,8 @@
  *             P.post_batch = b (optional, 0 = off; -1: floor(sqrt(n)), b >= 1: batch length b; needs post_levels)
  *             adds batch_mean, batch_within, batch_between, half_mean, half_within, half_between, batch_len,
  *             n_batches, half_n, ESS, MCSE, Rhat_split to each (sbd_posterior_diagnostics)
+ *             P.post_ci = alpha (optional, 0 = off; 0 < alpha < 1; needs post_levels) adds ci_alpha, ci_count, lower,
+ *             median, upper, ci_width (the 1 - alpha credible interval and the median, sbd_posterior_quantiles)
  *   [v,k]   = sbd_mex('max_eigenval', [M N], model, t, phi, psi, tol, maxit, x0)   utils/max_eigenval_*.m
  *   [y,s,n] = sbd_mex('observe', x, model, t, phi, psi, bsnr, noise)      run_Gaussian_demo.m:145-168
  *   [x,obj,dist,mses] = sbd_mex('salsa', y, model, t, phi, psi, tau, mu, maxiter, tolA, tviters, xtrue)
@@ -108,20 +110,25 @@ static mxArray* vec(int n, double** p) {
 }
 
 /* posterior statistics of the last run at block sizes 1 .. 2^(levels-1), with var, std and Rhat formed as DESIGN.md
-   states them ("Posterior statistics"); diag: also the diagnostics with ESS, MCSE and Rhat_split */
-static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels, int diag) {
+   states them ("Posterior statistics"); diag: also the diagnostics with ESS, MCSE and Rhat_split; ci: also the
+   credible interval and the median */
+static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels, int diag, int ci) {
     static const char* fields[] = {"scale", "n", "chains", "mean", "within", "between", "var", "std", "Rhat",
                                    "batch_mean", "batch_within", "batch_between", "half_mean", "half_within",
                                    "half_between", "batch_len", "n_batches", "half_n", "ESS", "MCSE", "Rhat_split"};
+    static const char* qfields[] = {"ci_alpha", "ci_count", "lower", "median", "upper", "ci_width"};
+    const char* names[27];
     char lnames[8][8];
     const char* lp[8];
     mxArray* out;
-    int j, rc;
+    int j, rc, nf = 0;
+    for (j = 0; j < (diag ? 21 : 9); ++j) names[nf++] = fields[j];
+    for (j = 0; ci && j < 6; ++j) names[nf++] = qfields[j];
     for (j = 0; j < levels; ++j) { snprintf(lnames[j], sizeof lnames[j], "s%d", 1 << j); lp[j] = lnames[j]; }
     out = mxCreateStructMatrix(1, 1, levels, lp);
     for (j = 0; j < levels; ++j) {
         const int s = 1 << j, bx = (rows + s - 1) / s, by = (cols + s - 1) / s;
-        mxArray* e = mxCreateStructMatrix(1, 1, diag ? 21 : 9, fields);
+        mxArray* e = mxCreateStructMatrix(1, 1, nf, names);
         mxArray *a[6];
         double* p[6];
         int q, n = 0, C = 0;
@@ -160,6 +167,23 @@ static mxArray* posterior_struct(sbd_ctx* c, int rows, int cols, int levels, int
             mxSetField(e, 0, "n_batches", mxCreateDoubleScalar((double)B));
             mxSetField(e, 0, "half_n", mxCreateDoubleScalar((double)h));
             mxSetField(e, 0, "ESS", d[6]); mxSetField(e, 0, "MCSE", d[7]); mxSetField(e, 0, "Rhat_split", d[8]);
+        }
+        if (ci) {
+            mxArray* u[4];
+            double* g[4];
+            double alpha = 0.0;
+            long long count = 0;
+            for (q = 0; q < 4; ++q) { u[q] = mxCreateDoubleMatrix(bx, by, mxREAL); g[q] = mxGetPr(u[q]); }
+            rc = sbd_posterior_quantiles(c, j, g[0], g[1], g[2], &alpha, &count);
+            if (rc) {
+                sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); sbd_set_posterior_quantiles(c, 0.0);
+                fail(c, "sbd_posterior_quantiles", rc);
+            }
+            for (i = 0; i < (size_t)bx * by; ++i) g[3][i] = g[2][i] - g[0][i];         /* ci_width */
+            mxSetField(e, 0, "ci_alpha", mxCreateDoubleScalar(alpha));
+            mxSetField(e, 0, "ci_count", mxCreateDoubleScalar((double)count));
+            mxSetField(e, 0, "lower", u[0]); mxSetField(e, 0, "median", u[1]); mxSetField(e, 0, "upper", u[2]);
+            mxSetField(e, 0, "ci_width", u[3]);
         }
         mxSetField(out, 0, lp[j], e);
     }
@@ -259,6 +283,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         sbd_ctx* c;
         double* q[21];
         int i, nm, levels, batch;
+        double ci;
         mxArray* r;
         if (!mxIsStruct(P)) mexErrMsgIdAndTxt("sbd:type", "P must be a struct");
         memset(&p, 0, sizeof p); memset(&t, 0, sizeof t);
@@ -281,6 +306,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         p.use_graph = (int)field(P, "use_graph", 0, -1);            /* -1: automatic (CUDA graph for small problems) */
         levels = (int)field(P, "post_levels", 0, 0);                 /* posterior statistics, 0 = off */
         batch = (int)field(P, "post_batch", 0, 0);                   /* their diagnostics, 0 = off */
+        ci = field(P, "post_ci", 0, 0);                              /* credible level alpha, 0 = off */
         c = get_ctx(rows, cols, (int)mxGetScalar(prhs[5]), (int)mxGetScalar(prhs[4]), mxGetScalar(prhs[6]), p.n_chains);
         nm = p.samples - p.burnIn; if (nm < 0) nm = 0;
         /* the `posterior` field exists only when it was asked for: otherwise the old field set */
@@ -298,13 +324,20 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         { mxArray* a = mxCreateDoubleMatrix(rows, cols * p.n_chains, mxREAL); t.X_last = mxGetPr(a); mxSetField(r, 0, "X_last", a); }
         if ((rc = sbd_set_posterior(c, levels))) fail(c, "sbd_set_posterior", rc);
         if ((rc = sbd_set_posterior_diagnostics(c, batch))) { sbd_set_posterior(c, 0); fail(c, "sbd_set_posterior_diagnostics", rc); }
+        if ((rc = sbd_set_posterior_quantiles(c, ci))) {
+            sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); fail(c, "sbd_set_posterior_quantiles", rc);
+        }
         rc = sbd_sapg_run(c, y, X0, xt, &p, noise, &t);
-        if (rc) { sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); fail(c, "sbd_sapg_run", rc); }
+        if (rc) {
+            sbd_set_posterior(c, 0); sbd_set_posterior_diagnostics(c, 0); sbd_set_posterior_quantiles(c, 0.0);
+            fail(c, "sbd_sapg_run", rc);
+        }
         if (levels > 0) {
             mxArray* post;
-            post = posterior_struct(c, rows, cols, levels, batch != 0);
+            post = posterior_struct(c, rows, cols, levels, batch != 0, ci != 0.0);
             sbd_set_posterior(c, 0);                             /* cached context: the requests are sticky */
             sbd_set_posterior_diagnostics(c, 0);
+            sbd_set_posterior_quantiles(c, 0.0);
             mxSetField(r, 0, "posterior", post);
         }
         { double* e; mxSetField(r, 0, "EB", vec(4, &e)); for (i = 0; i < 4; ++i) e[i] = t.EB[i]; }

@@ -86,13 +86,17 @@ class ChainShard:
         var, std and Rhat recomputed from the merged statistics.
         With the diagnostics (Engine.sapg(..., post_batch=b)) the batch statistics are merged the same way with
         weights C_r and the half statistics with weights 2 C_r, and ESS, MCSE and Rhat_split are recomputed; the
-        ranks must agree in n, batch_len and n_batches."""
+        ranks must agree in n, batch_len and n_batches.
+        Quantiles (Engine.sapg(..., post_ci=alpha)) do not merge: each rank's P^2 markers summarise the stream of its
+        own chains, and marker states of different streams give no estimator of the pooled one.  One rank passes them
+        through; with more than one, results that carry them raise ValueError on every rank."""
         from .host import posterior_moments, posterior_diagnostics
         out = []
         for st in stats:
             diag = "batch_mean" in st
             keys = ("mean", "within", "between") + (DIAG_KEYS if diag else ())
             local = np.stack([np.asarray(st[k], dtype=np.float64) for k in keys])
+            quant = "median" in st
             meta = [int(st["chains"]), int(st["n"]), int(diag)]
             if diag:
                 meta += [int(st["batch_len"]), int(st["n_batches"]), int(st["half_n"])]
@@ -101,10 +105,14 @@ class ChainShard:
             else:
                 import torch
                 import torch.distributed as dist
-                mt = torch.tensor(meta + [0] * (6 - len(meta)), dtype=torch.int64)
+                mt = torch.tensor(meta + [0] * (6 - len(meta)) + [int(quant)], dtype=torch.int64)
                 mts = [torch.empty_like(mt) for _ in range(self.world_size)]
                 dist.all_gather(mts, mt)
                 metas = [[int(v) for v in m] for m in mts]
+                if any(m[6] for m in metas):
+                    raise ValueError("combine_posterior: posterior quantiles (post_ci) cannot be merged across ranks: "
+                                     "the P^2 markers of each rank's chains give no estimator of the pooled stream; "
+                                     "hold all chains on one context (one rank) to get credible intervals")
                 if len({m[2] for m in metas}) != 1:
                     raise ValueError("combine_posterior: some ranks have diagnostics and some do not")
                 mine = torch.from_numpy(np.ascontiguousarray(local))
@@ -130,11 +138,14 @@ class ChainShard:
                 d.update(batch_len=b, n_batches=B, half_n=h)
                 d["ESS"], d["MCSE"], d["Rhat_split"] = posterior_diagnostics(
                     var, d["batch_within"], d["batch_between"], d["half_within"], d["half_between"], ns[0], C_, b, B, h)
+            if quant:                           # one rank (more were refused above)
+                d.update({k: st[k] for k in QUANT_KEYS})
             out.append(d)
         return out
 
 
 DIAG_KEYS = ("batch_mean", "batch_within", "batch_between", "half_mean", "half_within", "half_between")
+QUANT_KEYS = ("ci_alpha", "ci_count", "lower", "median", "upper", "ci_width")
 
 
 def _merge(counts, parts):
